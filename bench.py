@@ -66,7 +66,12 @@ def parse_args():
     ap.add_argument('--no-crop-gather', action='store_true', help='skip the separate crop-gather stage at N > 1')
     ap.add_argument('--gather-chunk', type=int, default=4096, help='uint8 crops per rank and chunk in the crop-gather stage')
     ap.add_argument('--gather-steps', type=int, default=8)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write what the last one computed to '
+                    'DIR/<name>.npy (float32 / float64, at most 64 MB; see OutputDump), e.g. DIR = bench_outputs')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 def workload_config(args, world=1, scenes_rank=None):
@@ -442,6 +447,57 @@ def extra_configs(args, torch, dev, images, images_h, peak, crops_buf):
     return out
 
 
+class OutputDump:
+    """--dump-outputs: what the timed path hands its caller in the last timed step, so that two builds run with the same
+    arguments can be compared file by file.
+
+    Per scene (all scenes while they fit in 14 MB, else a fixed seeded sample): the matcher's outputs idx, n, cost, X,
+    reproj and the scene's first ROI (scene_offset).  Per ROI (a fixed seeded sample that fits in 48 MB): the ROI
+    record, its status and its float32 crop.  The crops of a step never exist all at once (the pipeline reuses one
+    chunk buffer), so the sampled ones are copied out of each chunk as the pipeline hands it to its consumer.  Integer
+    arrays are written as float64 (exact); scene_index / roi_index say which rows were sampled."""
+
+    SCENE_BYTES, CROP_BYTES = 14_000_000, 48_000_000                    # + n_rois and the .npy headers: < 64 MB in all
+    SEED = 20251020
+
+    def __init__(self, torch, dev, S, Dmax, T, n_rois, chunk, crops):
+        def sample(n, k, stream):
+            if k >= n:
+                return np.arange(n)
+            return np.sort(np.random.default_rng([self.SEED, stream]).choice(n, k, replace=False))
+
+        self.torch, self.S = torch, S
+        per_scene = Dmax * 3 * 8 * 3 + Dmax * 4 + 3 * 8                  # idx, X, reproj; cost; n, scene_offset, scene_index
+        self.scenes = sample(S, self.SCENE_BYTES // per_scene, 0)
+        per_roi = 5 * 8 + 8 + (8 + 3 * T * T * 4 if crops else 0)       # ROI record, roi_index; status, crop
+        self.rois = sample(n_rois, self.CROP_BYTES // per_roi, 1)
+        self.crops = torch.empty((len(self.rois), 3, T, T), dtype=torch.float32, device=dev) if crops else None
+        self.parts = {}                                                  # chunk start -> (rows of self.crops, rows of the chunk)
+        for first in range(0, n_rois if crops else 0, chunk):
+            pos = np.flatnonzero((self.rois >= first) & (self.rois < first + chunk))
+            if len(pos):
+                self.parts[first] = (torch.as_tensor(pos, device=dev), torch.as_tensor(self.rois[pos] - first, device=dev))
+
+    def consumer(self, out, first):
+        part = self.parts.get(first)
+        if part is not None:
+            self.crops.index_copy_(0, part[0], out.index_select(0, part[1]))
+
+    def write(self, path, res, offs, rois, status):
+        torch = self.torch
+        sel = torch.as_tensor(self.scenes, device=offs.device)
+        ridx = torch.as_tensor(self.rois, device=offs.device)
+        arrays = {'scene_index': self.scenes, 'idx': res.idx[sel], 'n': res.n[sel], 'cost': res.cost[sel], 'X': res.X[sel],
+                  'reproj': res.reproj[sel], 'scene_offset': offs[sel], 'n_rois': offs[self.S:],
+                  'roi_index': self.rois, 'rois': rois[ridx]}
+        if self.crops is not None:
+            arrays.update(status=status[ridx], crops=self.crops)
+        os.makedirs(path, exist_ok=True)
+        for name, a in arrays.items():
+            a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+            np.save(os.path.join(path, f'{name}.npy'), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 def multi_rank_parity(args, torch, dist, dev, gathered, shards, Dmax, sample=64):
     """Rank 0: regenerate the first and the last `sample` scenes of every other rank's shard, run them locally and compare
     with the records that came through the all-gather, bit for bit (idx, n, cost, X, reproj)."""
@@ -486,6 +542,8 @@ def main():
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
     _guard_stdout()
+    if args.dump_outputs and world > 1:
+        raise SystemExit('--dump-outputs is supported at N = 1 only')
     if not torch.cuda.is_available():
         raise SystemExit('bench.py needs a CUDA device (there is no CPU fallback); use --impl reference for the CPU arm')
     torch.cuda.set_device(local)
@@ -532,15 +590,19 @@ def main():
         recbuf = torch.empty((distributed.records_bytes(S, Dmax),), dtype=torch.uint8, device=dev) if world > 1 else None
         gathered = torch.empty((world, recbuf.numel()), dtype=torch.uint8, device=dev) if world > 1 else None
 
-        def step(e=None):
+        def step(e=None, consumer=None):
             if e is not None:
                 e[3].record()
-            r, o = pipe.run_device(*tensors, n_rois_host=n_rois_arg, events=(e[0], e[1], e[2]) if e is not None else None)
+            r, o = pipe.run_device(*tensors, n_rois_host=n_rois_arg, events=(e[0], e[1], e[2]) if e is not None else None,
+                                   consumer=consumer)
             if world > 1:                 # final gather of the pose records over NVLink (SURVEY.md 8e): one pack kernel + one all-gather
                 distributed.gather_records(distributed.pack_records(r, o, 3, out=recbuf), out=gathered)
+            return r, o
         return step, gathered
 
-    def timed_loop(step, steps, warmup):
+    def timed_loop(step, steps, warmup, last_consumer=None):
+        """(ms, crop_ms, match_ms, wall0, wall1, (MatchResult, scene_offset) of the last step); ``last_consumer`` receives
+        the crop chunks of the last step."""
         ev = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(steps)]
         for _ in range(warmup):
             step()
@@ -552,7 +614,7 @@ def main():
         wall0 = time.time()
         t_start.record()
         for k in range(steps):
-            step(ev[k])
+            last = step(ev[k], consumer=last_consumer if k == steps - 1 else None)
         t_stop.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -565,21 +627,25 @@ def main():
             t = torch.tensor([ms, crop_ms, match_ms], dtype=torch.float64, device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms, crop_ms, match_ms = [float(v) for v in t.cpu()]
-        return ms, crop_ms, match_ms, wall0, wall1
+        return ms, crop_ms, match_ms, wall0, wall1, last
 
     step, gathered = make_step(pipe, (Ks, RTs, centers, counts, boxes, images, ios_d), n_rois_arg, S)
+    dump = (OutputDump(torch, dev, S, Dmax, T, n_rois, pipe.chunk, crops=not args.no_crops)
+            if args.dump_outputs else None)
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     launches0 = None
     warm = max(args.warmup, 3)
     for _ in range(warm):
-        step()
+        step(consumer=dump.consumer if dump else None)      # the dump's copy kernels load here, not in the timed window
     launches0 = _lib.launch_count()
-    ms, crop_ms, match_ms, wall0, wall1 = timed_loop(step, args.steps, 0)
+    ms, crop_ms, match_ms, wall0, wall1, last = timed_loop(step, args.steps, 0, dump.consumer if dump else None)
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     launches = _lib.launch_count() - launches0
     crop_launches = pipe.last_crop_launches * args.steps
+    if dump is not None:
+        dump.write(args.dump_outputs, *last, pipe.rois, pipe.status)
 
     # ---- N > 1: bit equality of what came through the gather, and the round-1 weak-scaling workload next to it ----
     parity = None
@@ -598,7 +664,7 @@ def main():
             _, offw = pipew.run_device(*tw)
             nw = int(offw[-1].item())
             stepw, _ = make_step(pipew, tw, nw, Sw)
-            msw, _, _, _, _ = timed_loop(stepw, 5, 3)
+            msw, _, _, _, _, _ = timed_loop(stepw, 5, 3)
             weak = {'workload': f'config 2 per rank: {Sw} scenes x {D} detections per GPU per step (weak scaling, the round-1 line)',
                     'value': world * Sw * 5 / (msw * 1e-3), 'unit': UNIT, 'ms_per_step': msw / 5, 'steps': 5, 'warmup': 3,
                     'crops_per_s': world * nw * 5 / (msw * 1e-3)}
