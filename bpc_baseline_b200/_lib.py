@@ -41,6 +41,7 @@ SIGNATURES = {
     'bpc_roi_crop_bf16': (_i, [_p, _i, _i, _i, _p, _i, _p, _i, _i, _p, _i, _p, _p, _p, _p, _sz, _p]),
     'bpc_normalise_lut': (_i, [_p, _p, _p, _p]),
     'bpc_crops_normalise': (_i, [_p, _p, _i, _i, _i, _p, _p, _p]),
+    'bpc_color_jitter': (_i, [_p, _i, _i, _p, _p, _i, _p, _p, _p]),
 }
 
 _lib = None

@@ -485,6 +485,39 @@ def crops_normalise(sources: Sequence[torch.Tensor], T: int, swap_rb: bool = Tru
     return out
 
 
+def color_jitter(canvases: torch.Tensor, order: torch.Tensor, factors: torch.Tensor, swap_rb: bool = False,
+                 lut: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """torchvision ColorJitter on ``Image.fromarray(canvas)`` + to_tensor + normalize, bit-exact, for n canvases at once.
+
+    ``canvases`` uint8 [n,T,T,3] (e.g. :func:`roi_crop_u8`; channel 0 is treated as PIL's R), ``order`` i32 [n,4] and
+    ``factors`` f32 [n,4] as drawn by ``utils.data_utils.draw_color_jitter``.  Returns f32 [n,3,T,T]; ``swap_rb`` and
+    ``lut`` as :func:`roi_crop` (the training dataset keeps the stored order: ``swap_rb=False``)."""
+    _chk(canvases, torch.uint8, 'canvases', 4); _chk(order, torch.int32, 'order', 2); _chk(factors, torch.float32, 'factors', 2)
+    n, T = canvases.shape[0], canvases.shape[1]
+    if tuple(canvases.shape[1:]) != (T, T, 3) or tuple(order.shape) != (n, 4) or tuple(factors.shape) != (n, 4):
+        raise RuntimeError('expected canvases [n,T,T,3], order [n,4] and factors [n,4]')
+    if not 1 <= T <= MAX_TARGET:
+        raise RuntimeError(f'target size must be in 1..{MAX_TARGET}')
+    dev = canvases.device
+    if order.device != dev or factors.device != dev:
+        raise RuntimeError('canvases, order and factors must be on the same device')
+    if lut is None:
+        lut = normalise_lut(dev)
+    _chk(lut, torch.float32, 'lut', 2)
+    if tuple(lut.shape) != (3, 256):
+        raise RuntimeError('lut must be [3,256]')
+    if out is None:
+        out = torch.empty((n, 3, T, T), dtype=torch.float32, device=dev)
+    else:
+        _chk(out, torch.float32, 'out', 4)
+        if out.shape[0] < n or tuple(out.shape[1:]) != (3, T, T):
+            raise RuntimeError('out must be [>=n,3,T,T]')
+    with torch.cuda.device(dev):
+        _lib.check(_lib.load().bpc_color_jitter(_p(canvases), n, T, _p(order), _p(factors), int(bool(swap_rb)), _p(lut), _p(out),
+                                                _stream(dev)), 'bpc_color_jitter')
+    return out
+
+
 def train_rois(xywh: torch.Tensor, W: int, H: int, image: Optional[torch.Tensor] = None, scale: Optional[torch.Tensor] = None,
                shift: Optional[torch.Tensor] = None) -> torch.Tensor:
     """ROI records i32 [n,5] of the dataset's crops (data_utils.py:243-271): the original window, or with ``scale``

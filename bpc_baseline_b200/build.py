@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libbpc_b200.so')
-SOURCES = ['api.cu', 'match.cu', 'crop.cu', 'crop_cta.cu', 'gather.cu']
+SOURCES = ['api.cu', 'match.cu', 'crop.cu', 'crop_cta.cu', 'gather.cu', 'jitter.cu']
 HEADERS = ['common.cuh', 'geometry.cuh', 'lsap.cuh', 'crop_common.cuh']
 ARCH = ['-gencode', 'arch=compute_100a,code=sm_100a']
 

@@ -220,6 +220,27 @@ std::tuple<Tensor, Tensor> roi_crop_u8_meta(const Tensor& images, const Tensor& 
     return {at::empty_symint({rois.sym_size(0), T, T, 3}, images.options()), at::empty_symint({rois.sym_size(0)}, rois.options())};
 }
 
+// ---- training-side ColorJitter + to_tensor + normalize (bpc/utils/data_utils.py, torchvision ColorJitter) -----------
+Tensor color_jitter(const Tensor& canvases, const Tensor& order, const Tensor& factors, bool swap_rb, const Tensor& lut) {
+    chk(canvases, at::kByte, "canvases", 4); chk(order, at::kInt, "order", 2); chk(factors, at::kFloat, "factors", 2); chk(lut, at::kFloat, "lut", 2);
+    const int64_t n = canvases.size(0), T = canvases.size(1);
+    TORCH_CHECK(canvases.size(2) == T && canvases.size(3) == 3 && order.size(0) == n && order.size(1) == 4 && factors.size(0) == n &&
+                factors.size(1) == 4, "expected canvases [n,T,T,3], order [n,4] and factors [n,4]");
+    TORCH_CHECK(T >= 1 && T <= BPC_MAX_TARGET, "target size must be in 1..", BPC_MAX_TARGET);
+    TORCH_CHECK(lut.size(0) == 3 && lut.size(1) == 256, "lut must be [3,256]");
+    TORCH_CHECK(order.device() == canvases.device() && factors.device() == canvases.device() && lut.device() == canvases.device(),
+                "canvases, order, factors and lut must be on the same device");
+    const c10::cuda::CUDAGuard guard(canvases.device());
+    Tensor out = at::empty({n, 3, T, T}, lut.options());
+    rc_check(bpc_color_jitter(canvases.data_ptr<uint8_t>(), (int)n, (int)T, order.data_ptr<int32_t>(), factors.data_ptr<float>(), swap_rb ? 1 : 0,
+                              lut.data_ptr<float>(), out.data_ptr<float>(), cur_stream(canvases)), "bpc_color_jitter");
+    return out;
+}
+
+Tensor color_jitter_meta(const Tensor& canvases, const Tensor&, const Tensor&, bool, const Tensor& lut) {
+    return at::empty_symint({canvases.sym_size(0), 3, canvases.sym_size(1), canvases.sym_size(2)}, lut.options());
+}
+
 // ---- pose records for the final gather (SURVEY.md 8e) --------------------------------------------------------------
 Tensor pack_records(const Tensor& idx, const Tensor& n, const Tensor& cost, const Tensor& X, const Tensor& reproj, const Tensor& scene_offset,
                     int64_t offset_div) {
@@ -258,6 +279,7 @@ TORCH_LIBRARY(bpc_b200, m) {
           "Tensor(a!)? out=None) -> (Tensor(a!), Tensor)");
     m.def("roi_crop_u8(Tensor images, Tensor rois, int T, int[] fill, Tensor? n_rois=None, int roi_first=0) -> (Tensor, Tensor)");
     m.def("roi_crop_bf16(Tensor images, Tensor rois, int T, int[] fill, bool swap_rb, Tensor lut, Tensor? n_rois=None, int roi_first=0) -> (Tensor, Tensor)");
+    m.def("color_jitter(Tensor canvases, Tensor order, Tensor factors, bool swap_rb, Tensor lut) -> Tensor");
     m.def("pack_records(Tensor idx, Tensor n, Tensor cost, Tensor X, Tensor reproj, Tensor scene_offset, int offset_div=3) -> Tensor");
     m.def("fundamental(Tensor Ks, Tensor RTs) -> Tensor");
     m.def("abi_version() -> int", &abi_version);
@@ -270,6 +292,7 @@ TORCH_LIBRARY_IMPL(bpc_b200, CUDA, m) {
     m.impl("roi_crop", &roi_crop);
     m.impl("roi_crop_u8", &roi_crop_u8);
     m.impl("roi_crop_bf16", &roi_crop_bf16);
+    m.impl("color_jitter", &color_jitter);
     m.impl("pack_records", &pack_records);
     m.impl("fundamental", &fundamental);
 }
@@ -281,4 +304,5 @@ TORCH_LIBRARY_IMPL(bpc_b200, Meta, m) {
     m.impl("roi_crop", &roi_crop_meta);
     m.impl("roi_crop_u8", &roi_crop_u8_meta);
     m.impl("roi_crop_bf16", &roi_crop_bf16_meta);
+    m.impl("color_jitter", &color_jitter_meta);
 }

@@ -83,6 +83,14 @@ def roi_crop_bf16(images, rois, T: int = 256, fill=(255, 255, 255), swap_rb: boo
     return load().roi_crop_bf16(images, rois, int(T), [int(v) for v in fill], bool(swap_rb), lut, n_rois, int(roi_first))
 
 
+def color_jitter(canvases, order, factors, swap_rb: bool = False, lut=None):
+    """f32 [n,3,T,T]: torchvision ColorJitter (draws of utils.data_utils.draw_color_jitter) + to_tensor + normalize on uint8
+    canvases [n,T,T,3], bit-exact (bpc_color_jitter)."""
+    if lut is None:
+        lut = normalise_lut(canvases.device)
+    return load().color_jitter(canvases, order, factors, bool(swap_rb), lut)
+
+
 def pack_records(idx, n, cost, X, reproj, scene_offset, offset_div: int = 3):
     return load().pack_records(idx, n, cost, X, reproj, scene_offset, int(offset_div))
 

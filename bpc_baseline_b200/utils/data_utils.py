@@ -216,16 +216,39 @@ def draw_crop_jitter(bbox_visib, rnd=None):
     return scale, shift
 
 
-def dataset_crops(images, bbox_visib, image_index=None, target_size=256, jitter=None, as_uint8=False):
+def draw_color_jitter(n, brightness=None, contrast=None, saturation=None, hue=None):
+    """The draws ``torchvision.transforms.ColorJitter(brightness, contrast, saturation, hue)`` makes for n samples, in its
+    order: per sample ``ColorJitter.get_params`` (``torch.randperm(4)``, then one float32 ``uniform_`` per enabled op), so
+    seeding torch's global RNG reproduces the per-sample transform.  The ranges are normalised by ColorJitter's own
+    argument checks (None = the op is off).  Returns (order int32 [n, 4] = op ids in application order with disabled ops
+    as -1, factors float32 [n, 4] = (brightness, contrast, saturation, hue), NaN where an op is off) for
+    :func:`batched.color_jitter` or ``dataset_crops(color_jitter=...)``."""
+    from torchvision.transforms import ColorJitter
+    cj = ColorJitter(brightness=0 if brightness is None else brightness, contrast=0 if contrast is None else contrast,
+                     saturation=0 if saturation is None else saturation, hue=0 if hue is None else hue)
+    order = np.empty((int(n), 4), np.int32)
+    factors = np.empty((int(n), 4), np.float32)
+    for r in range(int(n)):
+        fn_idx, *fac = ColorJitter.get_params(cj.brightness, cj.contrast, cj.saturation, cj.hue)
+        order[r] = [int(k) if fac[int(k)] is not None else -1 for k in fn_idx]
+        factors[r] = [np.nan if f is None else f for f in fac]
+    return order, factors
+
+
+def dataset_crops(images, bbox_visib, image_index=None, target_size=256, jitter=None, as_uint8=False, color_jitter=None):
     """Batched crop transform of BOPSingleObjDataset.__getitem__ (data_utils.py:243-252, 282; jittered window :257-271).
 
     ``images`` uint8 [B, H, W, 3] BGR (NumPy or CUDA tensor), ``bbox_visib`` int [n, 4] = (x, y, w, h), ``jitter`` =
     None for the original crop or the (scale, shift) pair of :func:`draw_crop_jitter` for the augmented window.
     Returns the normalised float32 [n, 3, T, T] CUDA tensor in the dataset's channel order (BGR kept, no swap), or the
-    uint8 letterboxed images [n, T, T, 3] with ``as_uint8`` (what the reference hands to ColorJitter, which is not
-    built here).  Raises RuntimeError on an empty crop, as the reference (:247-248, :269-270).
+    uint8 letterboxed images [n, T, T, 3] with ``as_uint8``.  ``color_jitter`` = the (order, factors) pair of
+    :func:`draw_color_jitter` (NumPy arrays, or int32 / float32 CUDA tensors taken as they are): the canvases go through
+    torchvision's ColorJitter (on ``Image.fromarray(canvas)``, bit-exact) before to_tensor + normalize; it cannot be
+    combined with ``as_uint8``.  Raises RuntimeError on an empty crop, as the reference (:247-248, :269-270).
     """
     import torch
+    if color_jitter is not None and as_uint8:
+        raise ValueError('color_jitter produces the normalised float32 tensor; it cannot be combined with as_uint8')
     imgs = images if isinstance(images, torch.Tensor) else _host.to_dev(images, np.uint8)
     _, H, W, _ = imgs.shape
     xywh = _host.to_dev(np.asarray(bbox_visib).reshape(-1, 4), np.int32)
@@ -235,10 +258,14 @@ def dataset_crops(images, bbox_visib, image_index=None, target_size=256, jitter=
         scale, shift = _host.to_dev(jitter[0], np.float64), _host.to_dev(jitter[1], np.int32)
     rois = batched.train_rois(xywh, W, H, image=idx, scale=scale, shift=shift)
     status = torch.zeros(rois.shape[0], dtype=torch.int32, device=rois.device)
-    if as_uint8:
+    if as_uint8 or color_jitter is not None:
         out = batched.roi_crop_u8(imgs, rois, T=int(target_size), status=status)
     else:
         out = batched.roi_crop(imgs, rois, T=int(target_size), swap_rb=False, status=status)
     if int(status.sum().item()):
         raise RuntimeError('Empty crop for %s image' % ('augmented' if jitter is not None else 'original'))
+    if color_jitter is not None:
+        order, factors = (d if isinstance(d, torch.Tensor) and d.is_cuda else _host.to_dev(d, dt)
+                          for d, dt in zip(color_jitter, (np.int32, np.float32)))
+        out = batched.color_jitter(out, order, factors, swap_rb=False)
     return out

@@ -256,6 +256,24 @@ int bpc_normalise_lut(const float* mean_host3, const float* std_host3, float* lu
 int bpc_crops_normalise(const uint8_t* const* srcs, const int32_t* counts, int n_src, int T, int swap_rb,
                         const float* lut, float* out, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Training-side ColorJitter (SURVEY 8f rank 3): torchvision.transforms.ColorJitter on
+ * Image.fromarray(canvas), then to_tensor + normalize -- what BOPSingleObjDataset.__getitem__ does
+ * with the jittered canvas (bpc/utils/data_utils.py), bit-exact with Pillow's arithmetic.  The
+ * random draws stay on the host (torch's RNG stream, ColorJitter.get_params); this only applies them.
+ *   in       uint8 [n][T][T][3]   e.g. the output of bpc_roi_crop_u8; stored channel 0 is PIL's R
+ *   order    int32 [n][4]         op ids in application order: 0 brightness, 1 contrast, 2 saturation,
+ *                                 3 hue, -1 = no op; each id at most once per crop (not checked: a repeated
+ *                                 contrast would reuse the first one's mean)
+ *   factors  float [n][4]         (brightness, contrast, saturation, hue) as float32 values; entries of
+ *                                 ops absent from `order` are ignored (any value, NaN included)
+ *   swap_rb, lut                  as bpc_roi_crop (the dataset uses swap_rb = 0)
+ *   out      float [n][3][T][T]
+ * 1 <= T <= BPC_MAX_TARGET; no workspace.  Fast path: T % 4 == 0 and 16-byte aligned in / out.
+ */
+int bpc_color_jitter(const uint8_t* in, int n, int T, const int32_t* order, const float* factors, int swap_rb,
+                     const float* lut, float* out, void* stream);
+
 /* Number of kernel launches issued by this library since load (all entry points). */
 unsigned long long bpc_launch_count(void);
 
