@@ -143,14 +143,20 @@ struct Scene {
 
 // Fill pts / lines / lvalid of a scene from global memory.  All threads of the CTA call it; the
 // caller must __syncthreads() afterwards.  F = [3][9] (12, 13, 23), already in shared memory.
-__device__ inline void scene_load(Scene& sc, const double* F, const double* centers_scene, int nthreads, int tid) {
+// Returns true when this thread loaded a point with a coordinate that is not below 1e300 in magnitude, or a line with a
+// component that is not finite.  Without any such input no pair distance can be NaN: every line component is finite and
+// |a|, |b| <= 1 (or the sentinel / zero line), so no product in |a x + b y + c| overflows and no inf - inf can occur.
+__device__ inline bool scene_load(Scene& sc, const double* F, const double* centers_scene, int nthreads, int tid) {
     const int D = sc.Dmax;
     const int cnt[3] = {sc.N, sc.M, sc.P};
+    bool suspect = false;
     for (int e = tid; e < 3 * D; e += nthreads) {
         const int cam = e / D, d = e - cam * D;
         if (d < cnt[cam]) {
-            sc.pts[(size_t)e * 2 + 0] = centers_scene[(size_t)e * 2 + 0];
-            sc.pts[(size_t)e * 2 + 1] = centers_scene[(size_t)e * 2 + 1];
+            const double x = centers_scene[(size_t)e * 2 + 0], y = centers_scene[(size_t)e * 2 + 1];
+            sc.pts[(size_t)e * 2 + 0] = x;
+            sc.pts[(size_t)e * 2 + 1] = y;
+            suspect |= !(fabs(x) < 1e300) || !(fabs(y) < 1e300);
         }
     }
     // set -> (F index, transpose, camera of the point)
@@ -167,7 +173,10 @@ __device__ inline void scene_load(Scene& sc, const double* F, const double* cent
         double* dst = sc.lines + (size_t)e * 3;
         dst[0] = ok ? l[0] : 0.0; dst[1] = ok ? l[1] : 0.0; dst[2] = ok ? l[2] : 9999.0;
         sc.lvalid[e] = ok ? 1 : 0;
+        const double INF = __longlong_as_double(0x7ff0000000000000LL);
+        suspect |= !(fabs(dst[0]) < INF) || !(fabs(dst[1]) < INF) || !(fabs(dst[2]) < INF);
     }
+    return suspect;
 }
 
 // ---- DLT triangulation of one 3-view match (epipolar_matching.py:118-127) ---------------------------

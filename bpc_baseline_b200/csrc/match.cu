@@ -56,7 +56,7 @@ struct ExplicitCost {           // dense float32 [N*M][P]
 struct RowMin {
     float* cmin;   // [P] float32 cost of the best column
     int* rlo;      // [P] lowest column index r attaining it
-    int* cnt;      // [P] number of columns attaining it (float32 equality)
+    int* cnt;      // [P] number of columns attaining it (float32 equality); 0 when the minimum is +inf
 };
 
 __device__ __forceinline__ double warp_min_d(double v) {
@@ -144,6 +144,9 @@ __device__ void row_argmin(const Scene& sc, int k, double* sa, double* sb, short
     }
     cnt = warp_sum_i(cnt);
     rlo = warp_min_i(rlo);
+    // a +inf minimum: every column may round to +inf, not only those below the bound, so the count is unknown (0 = not
+    // an immediate sink; the augmenting-path search then finds no finite path, and SciPy reports infeasible)
+    if (!(cmin < __int_as_float(0x7f800000))) cnt = 0;
     if (lane == 0) { out.cmin[k] = cmin; out.cnt[k] = cnt; out.rlo[k] = rlo; }
     __syncwarp();
 }
@@ -239,6 +242,24 @@ __device__ void VirtualCost::scan_unassigned(const LsapState& st, int t, int nov
         }
         __syncwarp();                                          // the scratch is reused by this warp's next chain row
     }
+}
+
+// ------------------------------------------------------------------------------------------------------
+// NaN test of a scene's virtual cost tensor (only for scenes whose scene_load reported a suspect input)
+// ------------------------------------------------------------------------------------------------------
+// An entry is NaN iff one of its three pair distances is (they are >= 0 or NaN), so every pair of the three pair
+// matrices is tested, O(N*M + N*P + M*P) < 2^24 pairs (Dmax <= 2048).
+__device__ __forceinline__ int scene_has_nan_cost(const Scene& sc, int nthreads, int tid) {
+    const int M = sc.M, P = sc.P, nNM = sc.N * M, nNP = sc.N * P, nMP = M * P;
+    int nan = 0;
+    for (int e = tid; e < nNM + nNP + nMP; e += nthreads) {
+        double d;
+        if (e < nNM) d = sc.e12(e / M, e % M);
+        else if (e < nNM + nNP) d = sc.e13((e - nNM) / P, (e - nNM) % P);
+        else d = sc.e23((e - nNM - nNP) / P, (e - nNM - nNP) % P);
+        nan |= d != d;
+    }
+    return nan;
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -344,12 +365,16 @@ __global__ void __launch_bounds__(256, 2) bpc_match_kernel(const float* __restri
             if (tid == 0) nout[s] = 0;
             continue;
         }
-        scene_load(sc, ms.F, centers + (size_t)s * 3 * Dmax * 2, nth, tid);
+        const bool suspect = scene_load(sc, ms.F, centers + (size_t)s * 3 * Dmax * 2, nth, tid);
         const int NM = N * M;
         const int transposed = NM > P;                       // SciPy: transpose iff more rows than columns
         const int nr = transposed ? P : NM, nc = transposed ? NM : P;
         lsap_reset(ms.st, nr, nc, nth, tid);
-        __syncthreads();
+        // a non-finite (or huge) centre or line: SciPy rejects the cost tensor if any entry is NaN (BPC_N_INFEASIBLE)
+        if (__syncthreads_or(suspect) && __syncthreads_or(scene_has_nan_cost(sc, nth, tid))) {
+            if (tid == 0) nout[s] = BPC_N_INFEASIBLE;
+            continue;
+        }
         // ---- phase 1 ---------------------------------------------------------------------------------
         if (transposed) {
             const int w = warp_id();
@@ -387,8 +412,8 @@ __global__ void __launch_bounds__(256, 2) bpc_match_kernel(const float* __restri
             ++row;
         }
         __syncthreads();
-        if (st.ctl[2]) {                                     // infeasible (NaN / inf costs): SciPy raises
-            if (tid == 0) nout[s] = -1;
+        if (st.ctl[2]) {                                     // infeasible (a row of +inf costs): SciPy raises
+            if (tid == 0) nout[s] = BPC_N_INFEASIBLE;
             continue;
         }
         // ---- phase 3 ---------------------------------------------------------------------------------

@@ -103,7 +103,8 @@ int bpc_match_objects(const float* cost, int S, int N, int M, int P, float thres
  *              needs reproj != NULL.
  *   Kmax       = Dmax
  *   idx    int32  [S][Kmax][3]  matches sorted by (cost, r); -1 padded
- *   n      int32  [S]           matches per scene (0 if any camera has no detection, :161-163; BPC_N_INFEASIBLE;
+ *   n      int32  [S]           matches per scene (0 if any camera has no detection, :161-163; BPC_N_INFEASIBLE where
+ *                               SciPy raises: a NaN cost, e.g. from a NaN or infinite centre, or no feasible assignment;
  *                               BPC_N_OVERFLOW if a count exceeds Dmax -- never a silent empty result)
  *   cost   float  [S][Kmax]     cost of each match (NaN padded)
  *   X      double [S][Kmax][3]  triangulated points (NaN padded)

@@ -6,8 +6,7 @@ import pytest
 import torch
 
 from oracle import crop as ocrop
-from oracle import geometry as og
-from tests.gpu_util import batch_to_dev, rel_err, to_dev
+from tests.gpu_util import batch_to_dev, check_match_properties, oracle_map, rel_err, to_dev
 
 pytestmark = pytest.mark.gpu
 
@@ -20,65 +19,17 @@ def _match(batch, threshold=30):
     return {k: getattr(res, k).cpu().numpy() for k in ('idx', 'n', 'cost', 'X', 'reproj')}
 
 
-def _check_properties(batch, out, threshold=30.0, min_recovery=None):
-    idx, n, cost, X, reproj = out['idx'], out['n'], out['cost'], out['X'], out['reproj']
-    S, K, _ = idx.shape
-    cnt = batch.counts.astype(np.int64)
-    assert np.all(n >= 0) and np.all(n <= np.minimum(cnt[:, 0] * cnt[:, 1], cnt[:, 2]))   # min(N*M, P) assignments (F2)
-    slot = np.arange(K)[None, :]
-    valid = slot < n[:, None]
-    # padding / validity
-    assert np.all(idx[~valid] == -1) and np.all(np.isnan(cost[~valid]))
-    assert np.all(idx[valid] >= 0)
-    for c in range(3):
-        assert np.all(idx[..., c][valid] < np.broadcast_to(batch.counts[:, c:c + 1], (S, K))[valid])
-    # threshold and order: costs < threshold, non-decreasing; ties in ascending r = i*M + j (process_pose.py:183)
-    assert np.all(cost[valid] < np.float32(threshold))
-    c0, c1 = cost[:, :-1], cost[:, 1:]
-    both = valid[:, 1:]
-    assert np.all(c0[both] <= c1[both])
-    r = idx[..., 0].astype(np.int64) * batch.counts[:, 1:2] + idx[..., 1]
-    tie = both & (c0 == c1)
-    assert np.all(r[:, :-1][tie] < r[:, 1:][tie])
-    # a rectangular assignment: third-camera detections are used at most once, (i, j) pairs at most once
-    big = 1 << 40
-    kk = np.where(valid, idx[..., 2], -1 - slot).astype(np.int64)
-    assert all(len(np.unique(row)) == K for row in kk[:: max(1, S // 512)])
-    rr = np.where(valid, r, -big - slot)
-    assert all(len(np.unique(row)) == K for row in rr[:: max(1, S // 512)])
-    # triangulation: finite, and consistent with the detections (reprojection error of a 3-view DLT)
-    assert np.all(np.isfinite(X[valid])) and np.all(np.isfinite(reproj[valid]))
-    assert np.median(reproj[valid]) < 5.0
-    if min_recovery is not None:
-        s_ix = np.repeat(np.arange(S), K).reshape(S, K)
-        t0 = batch.truth[s_ix, 0, idx[..., 0].clip(min=0)]
-        t1 = batch.truth[s_ix, 1, idx[..., 1].clip(min=0)]
-        t2 = batch.truth[s_ix, 2, idx[..., 2].clip(min=0)]
-        same = (t0 == t1) & (t1 == t2) & (t0 >= 0)
-        assert same[valid].mean() >= min_recovery, same[valid].mean()
-
-
-def _oracle_scene(job):
-    Ks, RTs, cen = job
-    want = og.match_scene(Ks, RTs, cen, 30, cost_fn=og.cost_tensor_fast)
-    return want['idx'], want['cost'], want['X']
-
-
 def _check_against_oracle(batch, out, scenes):
     scenes = list(scenes)
     jobs = []
     for s in scenes:
         Ks, RTs = batch.capture_arrays(s)
         jobs.append((Ks, RTs, [batch.centers[s, c, :batch.counts[s, c]] for c in range(3)]))
-    if len(scenes) > 16:                      # a D = 200 scene costs the oracle ~0.3 s: fan the sample out over the host cores
-        import concurrent.futures as cf
-        import multiprocessing as mp
-        import os
-        with cf.ProcessPoolExecutor(min(16, len(os.sched_getaffinity(0))), mp_context=mp.get_context('spawn')) as pool:
-            wants = list(pool.map(_oracle_scene, jobs, chunksize=4))
-    else:
-        wants = [_oracle_scene(j) for j in jobs]
-    for s, (widx, wcost, wX) in zip(scenes, wants):
+    # a D = 200 scene costs the oracle ~0.3 s: fan a large sample out over the host cores
+    wants = oracle_map(jobs, 16 if len(scenes) > 16 else 1)
+    for s, want in zip(scenes, wants):
+        assert not isinstance(want, Exception), (s, want)
+        widx, wcost, wX = want['idx'], want['cost'], want['X']
         n = int(out['n'][s])
         assert n == len(widx) and np.array_equal(out['idx'][s, :n], widx), s
         if n:
@@ -91,7 +42,7 @@ def test_config2_batch_4096x20():
     batch = synth.make_scenes(4096, 20)
     out = _match(batch)
     assert int(out['n'].sum()) == 4096 * 20                      # clean scenes: every object matched
-    _check_properties(batch, out, min_recovery=0.99)
+    check_match_properties(batch, out, min_recovery=0.99)
     _check_against_oracle(batch, out, range(0, 4096, 256))
 
 
@@ -99,7 +50,7 @@ def test_config3_dense_bin_16384x200():
     from bpc_baseline_b200 import synth
     batch = synth.make_scenes(16384, 200)
     out = _match(batch)
-    _check_properties(batch, out, min_recovery=0.9)
+    check_match_properties(batch, out, min_recovery=0.9)
     assert out['n'].mean() > 190
     _check_against_oracle(batch, out, [0, 9999])
 
@@ -110,7 +61,7 @@ def test_config3_dense_bin_with_dropped_detections():
     from bpc_baseline_b200 import synth
     batch = synth.make_scenes(512, 200, p_drop=0.1, sigma=2.0, seed=synth.SEED + 31)
     out = _match(batch)
-    _check_properties(batch, out)
+    check_match_properties(batch, out)
     _check_against_oracle(batch, out, [0, 300])
 
 
@@ -123,7 +74,7 @@ def test_conflict_heavy_scenes_match_scipy(D, p_drop, sigma, n_dup, n_false, nsc
     from bpc_baseline_b200 import synth
     batch = synth.make_scenes(nscenes, D, p_drop=p_drop, sigma=sigma, n_dup=n_dup, n_false=n_false, seed=synth.SEED + 57)
     out = _match(batch)
-    _check_properties(batch, out)
+    check_match_properties(batch, out)
     _check_against_oracle(batch, out, range(nscenes))
 
 
@@ -137,7 +88,7 @@ def test_config5_131072_scenes_in_shards():
         out = _match(batch)
         total += int(out['n'].sum())
         if rank in (0, 7):
-            _check_properties(batch, out, min_recovery=0.99)
+            check_match_properties(batch, out, min_recovery=0.99)
             _check_against_oracle(batch, out, [0, hi - lo - 1])
     assert total == 131072 * 20
 
