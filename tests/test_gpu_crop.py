@@ -226,11 +226,12 @@ def test_long_roi_lists_are_split_into_launches(monkeypatch):
         assert np.array_equal(out[r].cpu().numpy().view(np.uint32), want.view(np.uint32))
 
 
-@pytest.mark.parametrize('T,swap', [(224, True), (256, False), (96, True)])
+@pytest.mark.parametrize('T,swap', [(224, True), (256, False), (96, True), (97, True), (100, False), (255, False)])
 def test_bf16_channels_last_variant_equals_rounded_float_tensor(T, swap):
     """bpc_roi_crop_bf16 (the pose head's input, process_pose.py:210-212): every value of the float32 tensor rounded to
     bfloat16 (round-to-nearest-even, what torch's .to(bfloat16) does), stored channels-last -- all regimes and classes,
-    a rejected box included; bit-equal to the float path's output after that rounding."""
+    a rejected box included; bit-equal to the float path's output after that rounding.  Odd T (97, 255) alternates the
+    crops' base between 4- and 2-byte alignment, T = 100 leaves a partial last strip."""
     from bpc_baseline_b200 import batched, synth
     images = to_dev(synth.make_images(3, seed=9))
     rng = np.random.default_rng([77, T])
