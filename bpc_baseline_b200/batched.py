@@ -33,6 +33,20 @@ def _chk(t: torch.Tensor, dtype, name: str, ndim: Optional[int] = None):
     return t
 
 
+def _chk_device(t: torch.Tensor, dev: torch.device, name: str):
+    if t.device != dev:
+        raise RuntimeError(f'{name}: on {t.device}, but the kernel runs on {dev}')
+    return t
+
+
+def _chk_lut(lut: torch.Tensor, dev: torch.device):
+    """The kernels read all 3 x 256 entries of the table from the device they run on."""
+    _chk(lut, torch.float32, 'lut', 2)
+    if tuple(lut.shape) != (3, 256):
+        raise RuntimeError(f'lut: shape {tuple(lut.shape)}, expected (3, 256)')
+    return _chk_device(lut, dev, 'lut')
+
+
 def _p(t: Optional[torch.Tensor]):
     return C.c_void_p(t.data_ptr()) if t is not None else None
 
@@ -374,13 +388,14 @@ def roi_crop(images: torch.Tensor, rois: torch.Tensor, T: int = 256, fill=(255, 
     dev = images.device
     if lut is None:
         lut = normalise_lut(dev)
-    _chk(lut, torch.float32, 'lut', 2)
+    _chk_lut(lut, dev)
     if out is None:
         out = torch.empty((R, 3, T, T), dtype=torch.float32, device=dev)
     else:
         _chk(out, torch.float32, 'out', 4)
         if out.shape[0] < R or tuple(out.shape[1:]) != (3, T, T):
             raise RuntimeError('out must be [>=R,3,T,T]')
+        _chk_device(out, dev, 'out')
     _chk_status(status, R)
     if n_rois is not None:
         _chk(n_rois, torch.int32, 'n_rois')
@@ -406,13 +421,14 @@ def roi_crop_bf16(images: torch.Tensor, rois: torch.Tensor, T: int = 256, fill=(
     dev = images.device
     if lut is None:
         lut = normalise_lut(dev)
-    _chk(lut, torch.float32, 'lut', 2)
+    _chk_lut(lut, dev)
     if out is None:
         out = torch.empty((R, 3, T, T), dtype=torch.bfloat16, device=dev, memory_format=torch.channels_last)
     else:
         if out.dtype != torch.bfloat16 or not out.is_cuda or out.dim() != 4 or out.shape[0] < R or tuple(out.shape[1:]) != (3, T, T) \
                 or not out.is_contiguous(memory_format=torch.channels_last):
             raise RuntimeError('out must be a channels_last bfloat16 CUDA tensor [>=R,3,T,T]')
+        _chk_device(out, dev, 'out')
     _chk_status(status, R)
     if n_rois is not None:
         _chk(n_rois, torch.int32, 'n_rois')
@@ -439,6 +455,7 @@ def roi_crop_u8(images: torch.Tensor, rois: torch.Tensor, T: int = 256, fill=(25
         _chk(out, torch.uint8, 'out', 4)
         if out.shape[0] < R or tuple(out.shape[1:]) != (T, T, 3):
             raise RuntimeError('out must be uint8 [>=R,T,T,3]')
+        _chk_device(out, dev, 'out')
     _chk_status(status, R)
     if n_rois is not None:
         _chk(n_rois, torch.int32, 'n_rois')
@@ -467,9 +484,11 @@ def crops_normalise(sources: Sequence[torch.Tensor], T: int, swap_rb: bool = Tru
         if tuple(s.shape[1:]) != (T, T, 3):
             raise RuntimeError('every source must be uint8 [n,T,T,3]')
     dev = torch.device(device) if device is not None else sources[0].device
+    if dev.type == 'cuda' and dev.index is None:
+        dev = torch.device('cuda', torch.cuda.current_device())
     if lut is None:
         lut = normalise_lut(dev)
-    _chk(lut, torch.float32, 'lut', 2)
+    _chk_lut(lut, dev)
     total = sum(int(s.shape[0]) for s in sources)
     if out is None:
         out = torch.empty((total, 3, T, T), dtype=torch.float32, device=dev)
@@ -477,6 +496,7 @@ def crops_normalise(sources: Sequence[torch.Tensor], T: int, swap_rb: bool = Tru
         _chk(out, torch.float32, 'out', 4)
         if out.shape[0] < total or tuple(out.shape[1:]) != (3, T, T):
             raise RuntimeError('out must be [>=sum(n_s),3,T,T]')
+        _chk_device(out, dev, 'out')
     ptrs = (C.c_void_p * len(sources))(*[s.data_ptr() if s.shape[0] else None for s in sources])
     counts = (C.c_int32 * len(sources))(*[int(s.shape[0]) for s in sources])
     with torch.cuda.device(dev):
@@ -503,15 +523,14 @@ def color_jitter(canvases: torch.Tensor, order: torch.Tensor, factors: torch.Ten
         raise RuntimeError('canvases, order and factors must be on the same device')
     if lut is None:
         lut = normalise_lut(dev)
-    _chk(lut, torch.float32, 'lut', 2)
-    if tuple(lut.shape) != (3, 256):
-        raise RuntimeError('lut must be [3,256]')
+    _chk_lut(lut, dev)
     if out is None:
         out = torch.empty((n, 3, T, T), dtype=torch.float32, device=dev)
     else:
         _chk(out, torch.float32, 'out', 4)
         if out.shape[0] < n or tuple(out.shape[1:]) != (3, T, T):
             raise RuntimeError('out must be [>=n,3,T,T]')
+        _chk_device(out, dev, 'out')
     with torch.cuda.device(dev):
         _lib.check(_lib.load().bpc_color_jitter(_p(canvases), n, T, _p(order), _p(factors), int(bool(swap_rb)), _p(lut), _p(out),
                                                 _stream(dev)), 'bpc_color_jitter')

@@ -265,3 +265,73 @@ def test_bf16_variant_refuses_unaligned_pools():
     with pytest.raises(RuntimeError):
         batched.roi_crop_bf16(images, rois, T=224)
     assert tuple(batched.roi_crop(images, rois, T=224).shape) == (1, 3, 224, 224)
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# argument checks of the batched crop API: a table or an output the kernels cannot use is refused before any launch
+# ----------------------------------------------------------------------------------------------------------------------
+class _NoLaunch:
+    """Stands in for libbpc_b200.so: reaching any entry point fails the test, so a wrapper that lets a bad argument
+    through fails here without a kernel ever reading or writing past a buffer."""
+
+    def __getattr__(self, name):
+        def entry(*args):
+            pytest.fail(f'{name} was called with arguments the wrapper must refuse')
+        return entry
+
+
+LUT_WRAPPERS = ('roi_crop', 'roi_crop_bf16', 'crops_normalise', 'color_jitter')
+OUT_WRAPPERS = LUT_WRAPPERS + ('roi_crop_u8',)
+
+
+def _call(name, lut_device='cuda:0', lut_shape=(3, 256), out_device='cuda:0', T=32):
+    from bpc_baseline_b200 import batched
+    images = torch.zeros((1, 64, 96, 3), dtype=torch.uint8, device='cuda:0')
+    rois = torch.tensor([[0, 4, 4, 60, 40]], dtype=torch.int32, device='cuda:0')
+    crops = torch.zeros((1, T, T, 3), dtype=torch.uint8, device='cuda:0')
+    lut = torch.zeros(lut_shape, dtype=torch.float32, device=lut_device)
+    out = torch.empty((1, 3, T, T), dtype=torch.float32, device=out_device)
+    if name == 'roi_crop':
+        return batched.roi_crop(images, rois, T=T, lut=lut, out=out)
+    if name == 'roi_crop_bf16':
+        out = out.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+        return batched.roi_crop_bf16(images, rois, T=T, lut=lut, out=out)
+    if name == 'roi_crop_u8':
+        return batched.roi_crop_u8(images, rois, T=T, out=torch.empty((1, T, T, 3), dtype=torch.uint8, device=out_device))
+    if name == 'crops_normalise':
+        return batched.crops_normalise([crops], T, lut=lut, out=out)
+    order = torch.tensor([[0, 1, 2, 3]], dtype=torch.int32, device='cuda:0')
+    factors = torch.ones((1, 4), dtype=torch.float32, device='cuda:0')
+    return batched.color_jitter(crops, order, factors, lut=lut, out=out)
+
+
+@pytest.mark.parametrize('shape', [(3, 128), (256, 3)])
+@pytest.mark.parametrize('name', LUT_WRAPPERS)
+def test_lut_of_another_shape_is_refused(monkeypatch, name, shape):
+    """A [3,128] table would be read 768 floats deep; a transposed [256,3] one would be read with the wrong layout."""
+    from bpc_baseline_b200 import _lib
+    monkeypatch.setattr(_lib, 'load', _NoLaunch)
+    with pytest.raises(RuntimeError, match=r'lut: shape'):
+        _call(name, lut_shape=shape)
+
+
+def test_crops_normalise_refuses_a_lut_off_its_device(monkeypatch):
+    """``device`` names where the kernel runs (its sources may be peer mappings); the table must be there."""
+    from bpc_baseline_b200 import _lib, batched
+    monkeypatch.setattr(_lib, 'load', _NoLaunch)
+    crops = torch.zeros((1, 32, 32, 3), dtype=torch.uint8, device='cuda:0')
+    lut = torch.zeros((3, 256), dtype=torch.float32, device='cuda:0')
+    with pytest.raises(RuntimeError, match=r'lut: on cuda:0, but the kernel runs on cuda:1'):
+        batched.crops_normalise([crops], 32, lut=lut, device='cuda:1')
+
+
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two GPUs')
+@pytest.mark.parametrize('name', OUT_WRAPPERS)
+def test_lut_and_out_off_the_launch_device_are_refused(monkeypatch, name):
+    from bpc_baseline_b200 import _lib
+    monkeypatch.setattr(_lib, 'load', _NoLaunch)
+    with pytest.raises(RuntimeError, match=r'out: on cuda:1, but the kernel runs on cuda:0'):
+        _call(name, out_device='cuda:1')
+    if name in LUT_WRAPPERS:
+        with pytest.raises(RuntimeError, match=r'lut: on cuda:1, but the kernel runs on cuda:0'):
+            _call(name, lut_device='cuda:1')

@@ -4,6 +4,9 @@ Bar: the float32 tensor rebuilt from gathered uint8 crops is bit-equal to what b
 which tests/test_gpu_crop.py pins bit-equal to the reference's cv2 + torchvision calls.
 """
 import os
+import re
+import signal
+import socket
 import subprocess
 import sys
 
@@ -77,13 +80,51 @@ def test_normalise_rejects_bad_arguments():
         batched.crops_normalise([u8], 32, out=torch.empty((1, 3, 32, 32), device='cuda'))
 
 
+def _free_port():
+    with socket.socket() as s:
+        s.bind(('127.0.0.1', 0))
+        return s.getsockname()[1]
+
+
+def _gather_check(nproc, transport, timeout=600):
+    """tools/gather_check.py --check under torchrun: (exit code, stdout, stderr).  torchrun and its workers run in a
+    session of their own, and the whole process group is killed when the run ends, so no worker outlives the test."""
+    env = dict(os.environ, PYTHONPATH=ROOT)
+    cmd = [sys.executable, '-m', 'torch.distributed.run', '--nnodes=1', f'--nproc-per-node={nproc}', '--master-addr',
+           '127.0.0.1', '--master-port', str(_free_port()), os.path.join(ROOT, 'tools', 'gather_check.py'),
+           '--transport', transport, '--check']
+    proc = subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, cwd=ROOT,
+                            start_new_session=True)
+    try:
+        out, err = proc.communicate(timeout=timeout)
+    except subprocess.TimeoutExpired:
+        os.killpg(proc.pid, signal.SIGKILL)
+        out, err = proc.communicate()
+        pytest.fail(f'gather_check did not finish in {timeout} s\n' + out[-2000:] + err[-4000:])
+    finally:
+        try:
+            os.killpg(proc.pid, signal.SIGKILL)
+        except ProcessLookupError:
+            pass
+    return proc.returncode, out, err
+
+
+def _assert_gathered(res):
+    code, out, err = res
+    assert code == 0, out[-2000:] + err[-4000:]
+    m = re.search(r'GATHER_OK chunks (\d+)', out)
+    assert m and int(m.group(1)) >= 5, out[-2000:]
+
+
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two GPUs')
 @pytest.mark.parametrize('transport', ['p2p', 'nccl'])
 def test_two_rank_crop_gather(transport):
     """tools/gather_check.py under torchrun: root's gathered tensor is bit-equal to direct crops of both shards."""
-    env = dict(os.environ, PYTHONPATH=ROOT)
-    cmd = [sys.executable, '-m', 'torch.distributed.run', '--nnodes=1', '--nproc-per-node=2', '--master-addr', '127.0.0.1',
-           '--master-port', '29541', os.path.join(ROOT, 'tools', 'gather_check.py'), '--transport', transport, '--check']
-    res = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
-    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-4000:]
-    assert 'GATHER_OK' in res.stdout
+    _assert_gathered(_gather_check(2, transport))
+
+
+@pytest.mark.parametrize('transport', ['nccl', 'p2p'])
+def test_one_rank_crop_gather(transport):
+    """The root's side of the gather on one GPU: its own chunks produced on the side stream, each slot reused at chunk
+    i + 2 after the conversion that read it (five chunks, the last ragged), against direct crops."""
+    _assert_gathered(_gather_check(1, transport))

@@ -4,7 +4,8 @@
         tools/gather_check.py --transport p2p --check --bench
 
 --check  root rebuilds every rank's ROIs locally, crops them directly (bpc_roi_crop) and compares bit for bit
-         with the tensor gathered from the ranks' uint8 crops; ragged last chunk included.  Prints GATHER_OK.
+         with the tensor gathered from the ranks' uint8 crops, over five chunks: both slots are reused (on the root
+         after waiting for the conversion that last read them) and the last chunk is ragged.  Prints GATHER_OK.
 --bench  times (a) produce + gather: every rank runs the uint8 crop kernel per chunk and the root collects;
          (b) gather only: the root collects chunks that are already in the ranks' buffers.  Device time
          (CUDA events on the root), one JSON line.
@@ -55,8 +56,8 @@ def main():
         print(f'transport {a.transport} peer mapping {cg.peers.method if cg.peers else None} world {world}', flush=True)
 
     if a.check:
-        n_check = min(chunk + chunk // 3, 600)                      # two chunks, the second ragged
         ck = min(chunk, 400)
+        n_check = 4 * ck + max(1, ck // 3)                          # five chunks, the last one ragged
         mine = torch.as_tensor(rank_rois(rank, n_check, B, H, W)).to(dev)
         ok = True
         for i, first in enumerate(range(0, n_check, ck)):
@@ -74,7 +75,7 @@ def main():
         flag = torch.tensor([1 if ok else 0], device=dev)
         dist.broadcast(flag, 0)
         if rank == 0:
-            print('GATHER_OK' if ok else 'GATHER_FAILED', flush=True)
+            print(f'GATHER_OK chunks {i + 1}' if ok else 'GATHER_FAILED', flush=True)
         if not int(flag.item()):
             cg.close()
             dist.destroy_process_group()
