@@ -161,7 +161,9 @@ def match_triangulate(Ks: torch.Tensor, RTs: torch.Tensor, centers: torch.Tensor
     """PoseEstimator._match (process_pose.py:144-188) for S scenes in one launch.
 
     ``reproj_thresh`` (pixels, default None = the reference's behaviour): drop every match whose reprojection error
-    (utils/triangulation.py:14-18) exceeds it in any view; the survivors keep their order.  ``n`` is negative for a
+    (utils/triangulation.py:14-18) exceeds it in any view; the survivors keep their order.  The test is ``error >
+    reproj_thresh``: an error equal to the threshold is kept, and so is a NaN error (NaN never exceeds it), e.g. a view
+    whose projection of X has w = 0 and a zero numerator.  ``n`` is negative for a
     scene SciPy would reject (-1) or whose counts exceed Dmax (-2): see :func:`check_match_status`."""
     _chk(Ks, torch.float32, 'Ks', 4); _chk(RTs, torch.float64, 'RTs', 4)
     _chk(centers, torch.float64, 'centers', 4); _chk(counts, torch.int32, 'counts', 2)

@@ -98,7 +98,8 @@ int bpc_match_objects(const float* cost, int S, int N, int M, int P, float thres
  *   threshold  compared as float32 against the float32 cost (epipolar_matching.py:110-111)
  *   has_reproj_thresh, reproj_thresh
  *              optional reprojection-error filter: with has_reproj_thresh != 0 a match is dropped when the error of ANY
- *              view exceeds reproj_thresh pixels; survivors keep their (cost, r) order, n is updated, the tail re-padded.
+ *              view exceeds reproj_thresh pixels (error > reproj_thresh: an equal or NaN error is kept); survivors keep
+ *              their (cost, r) order, n is updated, the tail re-padded.
  *              The reference has the helper but no call site that filters (SURVEY.md F7), so 0 = reference behaviour;
  *              needs reproj != NULL.
  *   Kmax       = Dmax
