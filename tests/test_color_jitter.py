@@ -174,16 +174,22 @@ def test_torch_op_is_registered_with_a_meta_kernel():
 
 # ---- the kernel against torchvision (GPU) ----------------------------------------------------------------------------
 
-def tv_tensor(canvas, order, factors, swap_rb=False):
-    """What ColorJitter.forward does with these draws (the _functional_pil ops in fn_idx order), then to_tensor +
-    normalize; swap_rb reverses the channels of the jittered image before to_tensor, as bpc_roi_crop's swap_rb."""
+def pil_jitter(canvas, order, factors):
+    """uint8 [T,T,3]: what ColorJitter.forward does with these draws (the _functional_pil ops in fn_idx order)."""
     import torchvision.transforms.functional as TF
     img = Image.fromarray(canvas)
     fns = (TF.adjust_brightness, TF.adjust_contrast, TF.adjust_saturation, TF.adjust_hue)
     for op in order:
         if op >= 0:
             img = fns[op](img, float(factors[op]))
-    arr = np.asarray(img)
+    return np.asarray(img)
+
+
+def tv_tensor(canvas, order, factors, swap_rb=False):
+    """pil_jitter, then to_tensor + normalize; swap_rb reverses the channels of the jittered image before to_tensor, as
+    bpc_roi_crop's swap_rb."""
+    import torchvision.transforms.functional as TF
+    arr = pil_jitter(canvas, order, factors)
     if swap_rb:
         arr = arr[..., ::-1].copy()
     return TF.normalize(TF.to_tensor(arr), MEAN, STD).numpy()
