@@ -17,16 +17,15 @@
 //                     box of eight source rows per ring slot, consumer warps = 32-column strips.  Classes 1 (regime
 //                     1, scale < 2, <= 3 taps per axis; scale exactly 1), 3 (regime 3) and 4 (regime 1 with 4..6 taps
 //                     per axis, 2 <= scale <= 5) and rejected boxes, whenever the image pitch is a multiple of 16
-//                     bytes and T <= 256;
-//   bpc_crop_warp     round 1's kernel, the path for other pitches / narrow images / T > 256: persistent CTAs, the
-//                     unit of work is (ROI, strip of 32 output columns), taken by ONE WARP from a global atomic
-//                     counter, plus one "padding" item per ROI; per-warp TMA staging (2-D boxes of four / eight rows,
-//                     or one 1-D bulk copy per row); walks its own list and exits at once when that is empty;
+//                     bytes, at least WARP_MAX_PITCH and cta_pitch_max(T), and T <= 256;
+//   bpc_crop_warp     the same classes on every other pool (other pitches, narrow images, T > 256): persistent CTAs,
+//                     the unit of work is (ROI, strip of 32 output columns), taken by ONE WARP from a global atomic
+//                     counter, plus one "padding" item per ROI; each warp stages its strip's source rows with one
+//                     1-D bulk copy per row (guarded cp.async for the last bytes of the pool);
 //   bpc_crop_generic  persistent CTAs over the (rare) remaining ROIs (class 2): integer ratios >= 2, scale > 5,
 //                     source rows streamed through shared memory in chunks (boxes as large as the image).
 // The dominant traffic is the float32 output (3*T*T*4 B per ROI): each warp stores 128 contiguous bytes per
 // plane and row; padding rows are written with 16-byte stores.
-#include <mutex>
 #include <type_traits>
 
 #include "crop_common.cuh"
@@ -44,8 +43,8 @@ constexpr int PREP_THREADS = BPC_PREP_THREADS;      // threads of a prep CTA (on
 // [h, hpad) stay zero (no contribution, no completed row) so that whole ring slots run to completion.  *bad is set when the taps
 // do not have this shape (then the ROI takes the generic path).
 __device__ void src_row_records(float2* ysrc, int cap, const RoiGeom& g, int maxtaps, int tid, int* bad) {
-    const int hpad = min(cap, ((g.h + STREAM_ROWS - 1) / STREAM_ROWS) * STREAM_ROWS + STREAM_ROWS);
-    if (g.h + STREAM_ROWS > cap) *bad = 1;
+    const int hpad = min(cap, ((g.h + CTA_ROWS - 1) / CTA_ROWS) * CTA_ROWS + CTA_ROWS);
+    if (g.h + CTA_ROWS > cap) *bad = 1;
     for (int s = tid; s < hpad; s += PREP_THREADS) ysrc[s] = make_float2(0.f, 0.f);
     __syncthreads();
     for (int d = tid; d < g.new_h && !*bad; d += PREP_THREADS) {
@@ -70,17 +69,18 @@ __device__ void src_row_records(float2* ysrc, int cap, const RoiGeom& g, int max
 // ------------------------------------------------------------------------------------------------------
 // Descriptor formats (float4; desc_stride(T) per ROI on the x axis, desc_stride(T) + 8 on the y axis):
 //   class 1 (area, <= 3 taps)  x: (w0, w1, w2, bits(first source column))
-//                              y: (b0, b1, b2, bits(first source row | taps << 24))          [image pitch not a multiple of 16]
-//                              y: float2 per SOURCE row s (the streaming path): (ba, bb).  |ba| = weight of row s in the
+//                              y: (b0, b1, b2, bits(first source row | taps << 24))          [warp kernel]
+//                              y: float2 per SOURCE row s [CTA kernel]: (ba, bb).  |ba| = weight of row s in the
 //                                 output row being accumulated; sign bit of ba set = that output row is complete after row s;
 //                                 bb = weight of row s as the first tap of the next output row (+0 if it has none there).
 //                                 An output row then is acc = (((0 + b0 h0) + b1 h1) + b2 h2), bit-identical to OpenCV's
 //                                 sum = b0 h0; sum += b1 h1; ... for non-negative terms.
 //   class 3 (fixed-point)      x: (bits(w0), bits(w1), 0, bits(source column))      w = 2048, 0 beyond xmax
 //                              y: (bits(b0), bits(b1), bits(second source row), bits(first source row))
-__global__ void __launch_bounds__(PREP_THREADS)
-bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, const int32_t* __restrict__ rois, int R,
-                     const int32_t* __restrict__ n_rois_dev, int roi_first, int T, int stream_ok,
+// Ten CTAs per SM (48 registers): left to itself ptxas 12.9 picks 50, which allocates as 56 and leaves room for nine
+__global__ void __launch_bounds__(PREP_THREADS, 10)
+bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, const int32_t* __restrict__ rois,
+                     const int32_t* __restrict__ n_rois_dev, int roi_first, int T, int use_cta,
                      RoiGeom* __restrict__ geom, float4* __restrict__ xdesc, float4* __restrict__ ydesc,
                      int32_t* __restrict__ glist, int32_t* __restrict__ gcount, int32_t* __restrict__ status, int32_t* __restrict__ list1) {
     __shared__ RoiGeom g;
@@ -132,8 +132,8 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
                         const int seg_px = (int)(31.0 * g.scale_x) + (int)ceil(g.scale_x) + 3;
                         const int pitch_max = ((3 * seg_px + 46) >> 4) << 4;
                         const bool taps6 = (int)ceil(g.scale_x) + 1 <= 6 && (int)ceil(g.scale_y) + 1 <= 6;
-                        // per-strip kernel: four ring slots of >= 2 rows fit 2 * WARP_BUF; CTA kernel (full-width rows): any width
-                        g.cls = (taps6 && ((stream_ok & 2) || pitch_max <= TMAP_MAX_PITCH)) ? 4 : 2;
+                        // warp kernel: a strip's rows fit its staging ring; CTA kernel (full-width rows): any width
+                        g.cls = (taps6 && (use_cta || pitch_max <= WARP_MAX_PITCH)) ? 4 : 2;
                     } else g.cls = 2;
                 }
             }
@@ -146,7 +146,7 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
     float4* yd = ydesc + (size_t)roi * ydesc_stride(T);
     if (cls == 4) {
         // (w_first, w_middle, w_last, bits(start | taps << 24)); a missing first / last tap takes the middle weight
-        for (int axis = 0; axis < ((stream_ok & 2) ? 1 : 2); ++axis) {
+        for (int axis = 0; axis < (use_cta ? 1 : 2); ++axis) {
             const int nd = axis ? g.new_h : g.new_w;
             for (int d = tid; d < nd; d += PREP_THREADS) {
                 int st, n, flags; float af, am, al;
@@ -156,7 +156,7 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
                 (axis ? yd : xd)[d] = make_float4(w0, am, wl, __int_as_float(st | (n << 24)));
             }
         }
-        if (stream_ok & 2) {
+        if (use_cta) {
             src_row_records(reinterpret_cast<float2*>(yd), 2 * ydesc_stride(T), g, 6, tid, &s_bad);
             if (s_bad && tid == 0) { g.cls = 2; }
         }
@@ -166,15 +166,15 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
             area_taps3(d, g.scale_x, g.w, xs, xn, w0, w1, w2);
             xd[d] = make_float4(w0, w1, w2, __int_as_float(xs));
         }
-        if (!(stream_ok & 1)) {
+        if (use_cta) {
+            src_row_records(reinterpret_cast<float2*>(yd), 2 * ds + YSRC_PAD, g, 3, tid, &s_bad);
+            if (s_bad && tid == 0) { g.cls = 2; }
+        } else {
             for (int d = tid; d < g.new_h; d += PREP_THREADS) {
                 int ys, yn; float b0, b1, b2;
                 area_taps3(d, g.scale_y, g.h, ys, yn, b0, b1, b2);
                 yd[d] = make_float4(b0, b1, b2, __int_as_float(ys | (yn << 24)));
             }
-        } else {
-            src_row_records(reinterpret_cast<float2*>(yd), 2 * ds + YSRC_PAD, g, 3, tid, &s_bad);
-            if (s_bad && tid == 0) { g.cls = 2; }
         }
     } else if (cls == 3) {
         for (int d = tid; d < g.new_w; d += PREP_THREADS) {
@@ -193,11 +193,7 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
     __syncthreads();
     if (tid == 0) {
         if (g.cls == 2) glist[atomicAdd(gcount, 1)] = roi;
-        if (list1 != nullptr) {
-            // crops streamed by bpc_crop_cta_kernel from the front of the list, those of bpc_crop_warp_kernel from its back
-            if (g.cls == 0 || g.cls == 1 || g.cls == 3 || g.cls == 4) list1[atomicAdd(gcount + 8, 1)] = roi;
-            else if (g.cls != 2 && g.cls != -1) list1[R - 1 - atomicAdd(gcount + 9, 1)] = roi;      // (none today)
-        }
+        else if (use_cta && g.cls != -1) list1[atomicAdd(gcount + 8, 1)] = roi;     // classes 0, 1, 3, 4: the CTA kernel's list
         geom[roi] = g;
     }
 }
@@ -245,30 +241,16 @@ __device__ __forceinline__ int warp_stage(unsigned char* buf, unsigned buf_s, un
     return 0;
 }
 
-// The same through a 2-D tensor map: box i = rows [row + i*rb, +rb) x pitch bytes from word column xw, issued by lane i.
-__device__ __forceinline__ void warp_stage_2d(unsigned buf_s, unsigned bar_s, const CUtensorMap* map, int xw, int row, int count,
-                                              int pitch, int rb, int lane) {
-    const int nboxes = (count + rb - 1) / rb;
-    if (lane == 0) mbar_expect_tx(bar_s, (unsigned)(nboxes * rb * pitch));
-    __syncwarp();
-    if (lane < nboxes)
-        asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                     :: "r"(buf_s + (unsigned)(lane * rb * pitch)), "l"(map), "r"(xw), "r"(row + lane * rb), "r"(bar_s) : "memory");
-}
-
-// TT = compile-time target size (0: run-time T); ALIGNED = the image row pitch W*3 is a multiple of 16 bytes
+// TT = compile-time target size (0: run-time T)
 // SWAP = write the planes in R, G, B order from B, G, R sources (cv2.COLOR_BGR2RGB, process_pose.py:206)
-template <bool OUT_U8, int TT, bool ALIGNED, bool SWAP>
+template <bool OUT_U8, int TT, bool SWAP>
 __global__ void __launch_bounds__(256, 3)
 bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, const RoiGeom* __restrict__ geom,
                      const float4* __restrict__ xdesc, const float4* __restrict__ ydesc, int32_t* __restrict__ wcount,
                      int R, int Trt, int nslot, uchar4 fill, int swap_rb, const float* __restrict__ lut_g,
-                     float* __restrict__ outf, uint8_t* __restrict__ outb, const __grid_constant__ TmapSet tm, const int32_t* __restrict__ wlist) {
+                     float* __restrict__ outf, uint8_t* __restrict__ outb) {
     extern __shared__ __align__(128) unsigned char smem[];
     float* lut = reinterpret_cast<float*>(smem);                                 // [3][LUT_STRIDE]: 256 values + the fill value
-    // wlist: the crops of this kernel, stored from the back of the list (the others belong to bpc_crop_cta_kernel); null = all of them
-    const int nmine = wlist ? wcount[5] : R;
-    if (nmine == 0) return;
     const int T = TT ? TT : Trt;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     unsigned char* wbase = smem + LUT_SMEM + wid * WARP_SMEM;         // [2][WARP_BUF] staging, then [2][32] float4 row descriptors
@@ -295,7 +277,7 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
     const unsigned long long img_end = (unsigned long long)(uintptr_t)images + (unsigned long long)B * H * rowstride;
     const float nz = __int_as_float((int)(0x80000000u | (unsigned)fill.w));     // -0.0f: fill.w is 0 at run time
     const u64 nz2 = pack2(nz, nz);
-    const long long nitems = (long long)nmine * nslot;
+    const long long nitems = (long long)R * nslot;
 
     for (;;) {
         int item = 0;
@@ -304,8 +286,7 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
         if (item >= nitems) break;
         // ROI-major order: a ROI's strips and its (store-only) padding item run at about the same time, which keeps
         // whole output rows together in DRAM and blends store-bound with issue-bound work (padding items last: -8 %)
-        const int ri = item / nslot, slot = item - ri * nslot;
-        const int roi = wlist ? wlist[R - 1 - ri] : ri;
+        const int roi = item / nslot, slot = item - roi * nslot;
         const RoiGeom* gp = geom + roi;
         const int cls = gp->cls;
         if (cls == -1 || cls == 2) continue;
@@ -338,24 +319,19 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
         const int xs_min = -warp_max_i32(-xs);
         const int xe_max = warp_max_i32(xs + xn);
         const int seg_bytes = 3 * (xe_max - xs_min);
-        const int pitch_need = ((15 + seg_bytes + 8 + 15) >> 4) << 4;
-        const int pitch = ALIGNED ? tmap_pitch(pitch_need) : pitch_need;
-        const int rb = tmap_rows(pitch);                                  // rows per TMA box (ALIGNED)
-        const CUtensorMap* map = &tm.m[ALIGNED ? tmap_index(pitch) : 0];
+        const int pitch = ((15 + seg_bytes + 8 + 15) >> 4) << 4;
         const int nv = pitch >> 4;
         const int rpp = 32 / nv, lr = lane / nv, lv = lane - lr * nv;
         const unsigned long long src_seg = gp->src + 3ull * (unsigned long long)xs_min;
-        const int mis0 = (int)(src_seg & 15ull), misstep = ALIGNED ? 0 : (int)(rowstride & 15ull);
-        const int colc = 3 * (xs - xs_min) + (ALIGNED ? mis0 : 0);
-        const int colc4 = colc & ~3, shc = (colc & 3) * 8;
-        const int rows_fit = ALIGNED ? (WARP_BUF / pitch) / rb * rb : WARP_BUF / pitch;
-        // tensor coordinates of the strip's first staged byte: flattened image row and uint32 column
-        const unsigned long long seg_off = (src_seg & ~15ull) - (unsigned long long)(uintptr_t)images;
-        const int row0 = ALIGNED ? (int)(seg_off / rowstride) : 0;
-        const int xw = ALIGNED ? (int)((seg_off - (unsigned long long)row0 * rowstride) >> 2) : 0;
+        const int mis0 = (int)(src_seg & 15ull), misstep = (int)(rowstride & 15ull);
+        const int colc = 3 * (xs - xs_min);
+        // byte offset of the lane's first tap in source row s of a buffer staged from row s_lo on: warp_stage() copies every
+        // row from the 16-byte boundary below its first byte, so the row's own misalignment moves the tap
+        auto tap_off = [&](int s, int s_lo) { return (s - s_lo) * pitch + colc + ((mis0 + s * misstep) & 15); };
+        const int rows_fit = WARP_BUF / pitch;
         const double scale_y = gp->scale_y;
-        // bh output rows tap at most bh*scale + 2 source rows; whole TMA boxes round that up by rb - 1 more
-        const int bh = max(1, min(32, (int)((double)(rows_fit - (ALIGNED ? 5 : 3)) / (scale_y < 1.0 ? 1.0 : scale_y))));
+        // bh output rows tap at most bh*scale + 2 source rows
+        const int bh = max(1, min(32, (int)((double)(rows_fit - 3) / (scale_y < 1.0 ? 1.0 : scale_y))));
         const int nb = (new_h + bh - 1) / bh;
         const float4* ydr = ydesc + (size_t)roi * ystride;
         float* optr = outf + ((size_t)roi * 3 * T + dy0) * T + x;     // (plane 0, current row, column x)
@@ -375,13 +351,8 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
             }
             const int s_lo = __shfl_sync(0xffffffffu, lo, 0);
             const int s_hi = __shfl_sync(0xffffffffu, hi, cnt - 1);
-            if (ALIGNED) {
-                warp_stage_2d(wbase_s + k * WARP_BUF, bar_s + 8 * k, map, xw, row0 + s_lo, s_hi - s_lo + 1, pitch, rb, lane);
-                bulk_next = 1;
-            } else {
-                bulk_next = warp_stage(wbase + k * WARP_BUF, wbase_s + k * WARP_BUF, bar_s + 8 * k, src_seg, rowstride, img_end, s_lo,
-                                       s_hi - s_lo + 1, pitch, lane, lr, lv, rpp);
-            }
+            bulk_next = warp_stage(wbase + k * WARP_BUF, wbase_s + k * WARP_BUF, bar_s + 8 * k, src_seg, rowstride, img_end, s_lo,
+                                   s_hi - s_lo + 1, pitch, lane, lr, lv, rpp);
             return s_lo;
         };
         auto load_desc = [&](int b) -> float4 {
@@ -405,17 +376,14 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
             const int s_first = __float_as_int(ydr[0].w) & 0xffffff;
             const int ysn_last = __float_as_int(ydr[new_h - 1].w);
             const int s_end = (ysn_last & 0xffffff) + (ysn_last >> 24);          // one past the last source row
-            const int G = ALIGNED ? ((2 * WARP_BUF / pitch) >> 2) / rb * rb       // rows per slot: whole TMA boxes
-                                  : min(32, (2 * WARP_BUF / pitch) >> 2);       // (1-D copies: lane r issues row r)
+            const int G = min(32, (2 * WARP_BUF / pitch) >> 2);                  // rows per slot (lane r issues row r)
             const int ngroups = (s_end - s_first + G - 1) / G;
             const unsigned slot_bytes = (unsigned)(G * pitch);
             unsigned bulkmask = 0;
             auto issue = [&](int g) {
                 const int j = g & 3, lo = s_first + g * G;
-                int bulk = 1;
-                if (ALIGNED) warp_stage_2d(wbase_s + j * slot_bytes, bar_s + 8 * j, map, xw, row0 + lo, min(G, s_end - lo), pitch, rb, lane);
-                else bulk = warp_stage(wbase + j * slot_bytes, wbase_s + j * slot_bytes, bar_s + 8 * j, src_seg, rowstride, img_end,
-                                       lo, min(G, s_end - lo), pitch, lane, lr, lv, rpp);
+                const int bulk = warp_stage(wbase + j * slot_bytes, wbase_s + j * slot_bytes, bar_s + 8 * j, src_seg, rowstride, img_end,
+                                            lo, min(G, s_end - lo), pitch, lane, lr, lv, rpp);
                 bulkmask = (bulkmask & ~(1u << j)) | ((unsigned)bulk << j);
             };
             auto wait = [&](int g) {
@@ -433,24 +401,16 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
             float hc2 = 0.f;
             auto strip = [&](auto nt_c) {
                 constexpr int NT = decltype(nt_c)::value;
-                unsigned gbase = wbase_s + colc4 - (unsigned)(s_first * pitch);          // ALIGNED: row r of the group at gbase + r * pitch
                 auto hrow = [&](int row) {
-                    if (row >= gend) {
-                        do {
-                            __syncwarp();                   // every lane is done with slot gi & 3
-                            if (gi + 4 < ngroups) issue(gi + 4);
-                            ++gi;
-                            wait(gi);
-                            gend += G;
-                        } while (row >= gend);
-                        gbase = wbase_s + (unsigned)(gi & 3) * slot_bytes + colc4 - (unsigned)((gend - G) * pitch);
+                    while (row >= gend) {
+                        __syncwarp();                       // every lane is done with slot gi & 3
+                        if (gi + 4 < ngroups) issue(gi + 4);
+                        ++gi;
+                        wait(gi);
+                        gend += G;
                     }
-                    if (ALIGNED) {
-                        h_area_n<NT>(gbase + (unsigned)(row * pitch), shc, w, c, hc01, hc2);
-                    } else {
-                        const int a = (row - (gend - G)) * pitch + colc + ((mis0 + row * misstep) & 15);
-                        h_area_n<NT>(wbase_s + (unsigned)(gi & 3) * slot_bytes + (a & ~3), (a & 3) * 8, w, c, hc01, hc2);
-                    }
+                    const int a = tap_off(row, gend - G);
+                    h_area_n<NT>(wbase_s + (unsigned)(gi & 3) * slot_bytes + (a & ~3), (a & 3) * 8, w, c, hc01, hc2);
                 };
                 float4 d = ydr[0];
                 for (int y = 0; y < new_h; ++y) {
@@ -491,95 +451,13 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
             continue;
         }
 
-        if (ALIGNED && cls == 1) {
-            // ---------------- regime 1, <= 3 taps per axis (scale < 2): source rows stream in order ----------------
-            // Ring of 8-row slots (one 2-D TMA box + the 64 bytes of the eight rows' (ba, bb) records per slot, one mbarrier
-            // each, every slot but the one being read in flight); the horizontal pass of four rows is computed back to back
-            // (12 independent loads), then every row is added to the open output row with weight |ba|; a row whose record
-            // has the sign of ba set closes that output row (LUT, three 128-byte stores) and opens the next one with
-            // weight bb.  No per-output-row tap loop, no tap-count branches, every source row staged exactly once.
-            ColW cw;
-            cw.set(xd.x, xd.y, xd.z);
-            if (!active) {                               // beside the image: every row sums to 256 -> LUT entry 256 = fill
-                cw.w[0] = cw.w[1] = cw.w[2] = 0.f;
-                cw.c[0] = 256.f; cw.c[1] = cw.c[2] = 0.f;
-            }
-            const int nchunks = (gp->h + STREAM_ROWS - 1) / STREAM_ROWS;
-            const unsigned slot_bytes = (unsigned)(STREAM_ROWS * pitch);
-            const int nsl = min(4, (2 * WARP_BUF) / (int)slot_bytes);                   // >= 3 (pitch <= STREAM_MAX_PITCH)
-            const unsigned dring = wbase_s + 2 * WARP_BUF;                              // [4 slots][8 rows] float2
-            const unsigned long long ysrc = (unsigned long long)(uintptr_t)(ydesc + (size_t)roi * ystride);
-            const CUtensorMap* map8 = &tm.m8[min(tmap_index(pitch), N_TMAPS8 - 1)];
-            auto issue = [&](int c, int j) {
-                if (lane == 0) {
-                    mbar_expect_tx(bar_s + 8 * j, slot_bytes + 8u * STREAM_ROWS);
-                    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                                 :: "r"(wbase_s + (unsigned)j * slot_bytes), "l"(map8), "r"(xw), "r"(row0 + c * STREAM_ROWS), "r"(bar_s + 8 * j) : "memory");
-                    bulk_g2s(dring + 8u * STREAM_ROWS * j, ysrc + 8ull * STREAM_ROWS * c, 8u * STREAM_ROWS, bar_s + 8 * j);
-                }
-            };
-            __syncwarp();                                   // previous item finished with the buffers
-            for (int c = 0; c < min(nsl, nchunks); ++c) issue(c, c);
-            u64 acc01 = 0ull;
-            float acc2 = 0.f;
-            unsigned roff = 0;                                // element offset of the open output row from optr
-            int yout = 0;
-            const bool store_ok = (TT && TT % 32 == 0) || x < T;
-            int j = 0;
-            for (int c = 0; c < nchunks; ++c) {
-                mbar_wait(bar_s + 8 * j, (ph >> j) & 1u); ph ^= 1u << j;
-                const unsigned rbase = wbase_s + (unsigned)j * slot_bytes + colc4;
-#pragma unroll
-                for (int half = 0; half < STREAM_ROWS / 4; ++half) {
-                    const float4 dA = lds_f4(dring + 8u * STREAM_ROWS * j + 32u * half), dB = lds_f4(dring + 8u * STREAM_ROWS * j + 32u * half + 16);
-                    u64 h01[4];
-                    float h2[4];
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) h_area3(rbase + (unsigned)((4 * half + k) * pitch), shc, cw, h01[k], h2[k]);
-                    if (half == STREAM_ROWS / 4 - 1) {
-                        __syncwarp();                           // every lane has read slot j: refill it
-                        if (c + nsl < nchunks) issue(c + nsl, j);
-                    }
-                    const float ba[4] = {dA.x, dA.z, dB.x, dB.z}, bb[4] = {dA.y, dA.w, dB.y, dB.w};
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        const float wa = fabsf(ba[k]);
-                        acc01 = fadd2(acc01, fprod2(pack2(wa, wa), h01[k], nz2));
-                        acc2 = __fadd_rn(acc2, __fmul_rn(wa, h2[k]));
-                        if (__float_as_int(ba[k]) < 0) {            // output row complete
-                            float a0f, a1f;
-                            unpack2(acc01, a0f, a1f);
-                            if (OUT_U8) {
-                                if (active) out.px(roi, dy0 + yout, x, round_u8(a0f), round_u8(a1f), round_u8(acc2));
-                                else if (padlane) out.pad(roi, dy0 + yout, x);
-                                ++yout;
-                            } else {
-                                const unsigned l0 = lut_addr(a0f, lut_m), l1 = lut_addr(a1f, lut_m), l2 = lut_addr(acc2, lut_m);
-                                if (store_ok) {
-                                    float* o = optr + roff;
-                                    stg_out<0>(o, lds_f32(swap ? l2 : l0));
-                                    stg_out<1>(o + plane, lds_f32(l1 + 4 * LUT_STRIDE));
-                                    stg_out<2>(o + 2 * plane, lds_f32((swap ? l0 : l2) + 8 * LUT_STRIDE));
-                                }
-                                roff += (unsigned)T;
-                            }
-                            acc01 = fprod2(pack2(bb[k], bb[k]), h01[k], nz2);
-                            acc2 = __fmul_rn(bb[k], h2[k]);
-                        }
-                    }
-                }
-                j = (j + 1 == nsl) ? 0 : j + 1;
-            }
-            continue;
-        }
-
         __syncwarp();                                   // previous item finished with the buffers
         int s_lo_cur = stage(0, 0, load_desc(0));
         bulk_cur = bulk_next;
         float4 ydn = load_desc(1);
         int s_lo_next = 0;
 
-        if (!ALIGNED && cls == 1) {
+        if (cls == 1) {
             ColW cw;
             cw.set(xd.x, xd.y, xd.z);
             int crow = -1;
@@ -605,25 +483,19 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
                         dnx = lds_f4(ring + (r + 1) * 16);          // next row's descriptor in flight behind this row's arithmetic
                         const int ysn = __float_as_int(d.w);
                         const int ys = ysn & 0xffffff, n = ysn >> 24;
-                        // byte address of the lane's first tap in row ys; with a 16-byte-multiple image pitch the
-                        // word offset and the funnel shift are per-item constants (pitch is a multiple of 16)
-                        int a = (ys - s_lo_cur) * pitch + colc;
-                        if (!ALIGNED) a += (mis0 + ys * misstep) & 15;
-                        const unsigned a4 = ALIGNED ? cur + (ys - s_lo_cur) * pitch + colc4 : cur + (a & ~3);
-                        if (ys != crow) h_area3(a4, ALIGNED ? shc : (a & 3) * 8, cw, hc01, hc2);
+                        const int a = tap_off(ys, s_lo_cur);
+                        if (ys != crow) h_area3(cur + (a & ~3), (a & 3) * 8, cw, hc01, hc2);
                         u64 acc01 = fprod2(pack2(d.x, d.x), hc01, nz2);
                         float acc2 = __fmul_rn(d.x, hc2);
                         if (n > 1) {
-                            int a1 = a + pitch;
-                            if (!ALIGNED) a1 = (ys + 1 - s_lo_cur) * pitch + colc + ((mis0 + (ys + 1) * misstep) & 15);
-                            h_area3(ALIGNED ? a4 + pitch : cur + (a1 & ~3), ALIGNED ? shc : (a1 & 3) * 8, cw, hc01, hc2);
+                            const int a1 = tap_off(ys + 1, s_lo_cur);
+                            h_area3(cur + (a1 & ~3), (a1 & 3) * 8, cw, hc01, hc2);
                             acc01 = fadd2(acc01, fprod2(pack2(d.y, d.y), hc01, nz2));
                             acc2 = __fadd_rn(acc2, __fmul_rn(d.y, hc2));
                         }
                         if (n > 2) {
-                            int a2 = a + 2 * pitch;
-                            if (!ALIGNED) a2 = (ys + 2 - s_lo_cur) * pitch + colc + ((mis0 + (ys + 2) * misstep) & 15);
-                            h_area3(ALIGNED ? a4 + 2 * pitch : cur + (a2 & ~3), ALIGNED ? shc : (a2 & 3) * 8, cw, hc01, hc2);
+                            const int a2 = tap_off(ys + 2, s_lo_cur);
+                            h_area3(cur + (a2 & ~3), (a2 & 3) * 8, cw, hc01, hc2);
                             acc01 = fadd2(acc01, fprod2(pack2(d.z, d.z), hc01, nz2));
                             acc2 = __fadd_rn(acc2, __fmul_rn(d.z, hc2));
                         }
@@ -672,7 +544,7 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
                         if (sy0 != rowA) {
                             if (sy0 == rowB) { HA[0] = HB[0]; HA[1] = HB[1]; HA[2] = HB[2]; }
                             else {
-                                const int a = (sy0 - s_lo_cur) * pitch + colc + (ALIGNED ? 0 : ((mis0 + sy0 * misstep) & 15));
+                                const int a = tap_off(sy0, s_lo_cur);
                                 h_lin(cur + (a & ~3), (a & 3) * 8, xw0, xw1, HA);
                             }
                             rowA = sy0;
@@ -680,7 +552,7 @@ bpc_crop_warp_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
                         if (sy1 != rowB) {
                             if (sy1 == rowA) { HB[0] = HA[0]; HB[1] = HA[1]; HB[2] = HA[2]; }
                             else {
-                                const int a = (sy1 - s_lo_cur) * pitch + colc + (ALIGNED ? 0 : ((mis0 + sy1 * misstep) & 15));
+                                const int a = tap_off(sy1, s_lo_cur);
                                 h_lin(cur + (a & ~3), (a & 3) * 8, xw0, xw1, HB);
                             }
                             rowB = sy1;
@@ -921,54 +793,6 @@ __global__ void bpc_lut_kernel(float m0, float m1, float m2, float s0, float s1,
     lut[t] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, 255.f), mean), sd);
 }
 
-// Tensor maps of the image pool for every staging pitch (host side, cached for the last pool seen).  The driver entry
-// point is fetched through the runtime, so the library still links against cudart only.
-static int tensor_maps(const uint8_t* images, int B, int H, int W, bool aligned, TmapSet* out) {
-    typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                 const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                 CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static std::mutex mu;
-    static TmapSet cached;
-    static const uint8_t* k_images = nullptr;
-    static int k_B = 0, k_H = 0, k_W = 0, k_dev = -1;
-    static EncodeFn encode = nullptr;
-    std::lock_guard<std::mutex> lock(mu);
-    if (!aligned) { memset(out, 0, sizeof(TmapSet)); return BPC_OK; }      // the 1-D bulk-copy variants ignore the maps
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (images == k_images && B == k_B && H == k_H && W == k_W && dev == k_dev) { *out = cached; return BPC_OK; }   // copied under the lock
-    if (!encode) {
-        cudaDriverEntryPointQueryResult q;
-        void* fnp = nullptr;
-        cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fnp, cudaEnableDefault, &q);
-        if (e != cudaSuccess) return (int)e;
-        if (q != cudaDriverEntryPointSuccess || !fnp) return (int)cudaErrorNotSupported;
-        encode = (EncodeFn)fnp;
-    }
-    const cuuint64_t gdim[2] = {(cuuint64_t)W * 3 / 4, (cuuint64_t)B * H};
-    const cuuint64_t gstride[1] = {(cuuint64_t)W * 3};
-    const cuuint32_t estr[2] = {1, 1};
-    for (int i = 0; i < N_TMAPS; ++i) {
-        const int pitch = i < 13 ? 64 + 32 * i : 512 + 64 * (i - 13);
-        const cuuint32_t box[2] = {(cuuint32_t)pitch / 4, (cuuint32_t)tmap_rows(pitch)};
-        const CUresult r = encode(&cached.m[i], CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, (void*)images, gdim, gstride, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, BPC_L2_PROMO,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { k_images = nullptr; return (int)cudaErrorInvalidValue; }
-    }
-    for (int i = 0; i < N_TMAPS8; ++i) {
-        const int pitch = 64 + 32 * i;
-        const cuuint32_t box[2] = {(cuuint32_t)pitch / 4, (cuuint32_t)STREAM_ROWS};
-        const CUresult r = encode(&cached.m8[i], CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, (void*)images, gdim, gstride, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, BPC_L2_PROMO,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { k_images = nullptr; return (int)cudaErrorInvalidValue; }
-    }
-    k_images = images; k_B = B; k_H = H; k_W = W; k_dev = dev;
-    *out = cached;
-    return BPC_OK;
-}
-
 // workspace: geom[R] | xdesc[R][ds] | ydesc[R][ydesc_stride(T)] | counters[16] | glist[R] | list1[R]    (ds = desc_stride(T), float4 records)
 static size_t ws_off_xdesc(int R) { return (((size_t)R * sizeof(RoiGeom)) + 15) & ~(size_t)15; }
 static size_t ws_off_ydesc(int R, int T) { return ws_off_xdesc(R) + (size_t)R * desc_stride(T) * sizeof(float4); }
@@ -991,42 +815,33 @@ static int launch_crop(const uint8_t* images, int B, int H, int W, const int32_t
     RoiGeom* geom = (RoiGeom*)wsb;
     float4* xdesc = (float4*)(wsb + ws_off_xdesc(R));
     float4* ydesc = (float4*)(wsb + ws_off_ydesc(R, T));
-    int32_t* gcount = (int32_t*)(wsb + ws_off_count(R, T));   // [0] generic-list length, [4] warp-item counter, [8] class-1 list length, [12] its work counter
+    int32_t* gcount = (int32_t*)(wsb + ws_off_count(R, T));   // [0] generic-list length, [4] warp-item counter, [8] CTA-list length, [12] its work counter
     int32_t* wcount = gcount + 4;
     int32_t* glist = gcount + 16;
     int32_t* list1 = glist + R;
     cudaError_t e = cudaMemsetAsync(gcount, 0, 64, st);
     if (e != cudaSuccess) return (int)e;
-    // 2-D TMA staging needs a 16-byte image pitch; rows narrower than the widest box keep the 1-D path
-    const bool aligned = ((long long)W * 3) % 16 == 0 && (long long)W * 3 >= TMAP_MAX_PITCH;
-    // class 1 through the warp-specialised CTA kernel: 2-D TMA staging, at most eight strips, full-width boxes inside the pool rows
-    const bool use_cta = aligned && T <= CTA_MAX_T && (long long)W * 3 >= cta_pitch_max(T);
+    // the CTA kernel stages full-width 2-D TMA boxes: a 16-byte row pitch, at most eight strips, its widest box inside the pool rows
+    const long long pitch = (long long)W * 3;
+    const bool use_cta = pitch % 16 == 0 && pitch >= WARP_MAX_PITCH && T <= CTA_MAX_T && pitch >= cta_pitch_max(T);
     if (BF16 && !use_cta) return BPC_EUNSUPPORTED;       // the bfloat16 output exists on the CTA kernel's path only
-    bpc_crop_prep_kernel<<<R, PREP_THREADS, 0, st>>>(images, B, H, W, rois, R, n_rois_dev, roi_first, T, (aligned ? 1 : 0) | (use_cta ? 2 : 0), geom, xdesc, ydesc,
-                                            glist, gcount, status, use_cta ? list1 : nullptr);
+    bpc_crop_prep_kernel<<<R, PREP_THREADS, 0, st>>>(images, B, H, W, rois, n_rois_dev, roi_first, T, use_cta ? 1 : 0, geom, xdesc, ydesc,
+                                            glist, gcount, status, list1);
     BPC_LAUNCH_CHECK();
     const uchar4 f4 = make_uchar4(fill[0], fill[1], fill[2], 0);
-    if (use_cta) {
+    if (use_cta) {                                        // every fast-class crop is on the CTA kernel's list
         const int rc = crop_cta_launch(OUT_U8 ? 1 : (BF16 ? 2 : 0), images, B, H, W, geom, xdesc, ydesc, list1, gcount, R, T, f4, swap_rb, lut,
                                        outf, outb, st);
         if (rc != BPC_OK) return rc;
-    }
-    if (!use_cta) {                                       // with the CTA kernel in use every fast-class crop is on ITS list
-        typedef void (*WarpFn)(const uint8_t*, int, int, int, const RoiGeom*, const float4*, const float4*, int32_t*, int, int, int,
-                               uchar4, int, const float*, float*, uint8_t*, const TmapSet, const int32_t*);
-        TmapSet tmaps;
-        const int terr = tensor_maps(images, B, H, W, aligned, &tmaps);
-        if (terr != BPC_OK) return terr;
-        WarpFn fn;
-        const bool sw = swap_rb != 0;
-#define BPC_PICK(TTV)                                                                                                  \
-    (aligned ? (sw ? bpc_crop_warp_kernel<OUT_U8, TTV, true, true> : bpc_crop_warp_kernel<OUT_U8, TTV, true, false>)   \
-             : (sw ? bpc_crop_warp_kernel<OUT_U8, TTV, false, true> : bpc_crop_warp_kernel<OUT_U8, TTV, false, false>))
-        if (OUT_U8) fn = aligned ? bpc_crop_warp_kernel<OUT_U8, 0, true, false> : bpc_crop_warp_kernel<OUT_U8, 0, false, false>;
-        else if (T == 224) fn = BPC_PICK(224);
-        else if (T == 256) fn = BPC_PICK(256);
-        else fn = BPC_PICK(0);
-#undef BPC_PICK
+    } else {
+        // the uint8 entry point never swaps channels and keeps T a run-time value: one variant
+        auto fn = bpc_crop_warp_kernel<OUT_U8, 0, false>;
+        if constexpr (!OUT_U8) {
+            const bool sw = swap_rb != 0;
+            if (T == 224) fn = sw ? bpc_crop_warp_kernel<false, 224, true> : bpc_crop_warp_kernel<false, 224, false>;
+            else if (T == 256) fn = sw ? bpc_crop_warp_kernel<false, 256, true> : bpc_crop_warp_kernel<false, 256, false>;
+            else if (sw) fn = bpc_crop_warp_kernel<false, 0, true>;
+        }
         // the same constant on every call: idempotent, so concurrent callers cannot interleave set(small) / launch(large)
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, WARPK_SMEM);
         if (e != cudaSuccess) return (int)e;
@@ -1039,24 +854,19 @@ static int launch_crop(const uint8_t* images, int B, int H, int W, const int32_t
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, cta_threads, WARPK_SMEM) != cudaSuccess || per_sm < 1) per_sm = 1;
         const long long slots = (long long)sms * per_sm;
         const int grid = (int)(want < slots ? want : slots);
-        fn<<<grid, cta_threads, WARPK_SMEM, st>>>(images, B, H, W, geom, xdesc, ydesc, wcount, R, T, nslot, f4, swap_rb, lut, outf, outb, tmaps, use_cta ? list1 : nullptr);
+        fn<<<grid, cta_threads, WARPK_SMEM, st>>>(images, B, H, W, geom, xdesc, ydesc, wcount, R, T, nslot, f4, swap_rb, lut, outf, outb);
         BPC_LAUNCH_CHECK();
     }
     const int nbands = (T + CROP_BAND - 1) / CROP_BAND;
     const long long max_items = (long long)R * nbands;
     const int grid = (int)(max_items < 148 * 2 ? max_items : 148 * 2);
     const int threads = ((T + 31) / 32) * 32;                   // one thread per output column
-    if (threads <= 256) {
-        e = cudaFuncSetAttribute(bpc_crop_generic_kernel<OUT_U8, 256, BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, CROP_RAW_BYTES);
-        if (e != cudaSuccess) return (int)e;
-        bpc_crop_generic_kernel<OUT_U8, 256, BF16><<<grid, threads, CROP_RAW_BYTES, st>>>(images, B, H, W, geom, glist, gcount, T, nbands, f4,
-                                                                                   swap_rb, lut, outf, outb);
-    } else {
-        e = cudaFuncSetAttribute(bpc_crop_generic_kernel<OUT_U8, 1024, BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, CROP_RAW_BYTES);
-        if (e != cudaSuccess) return (int)e;
-        bpc_crop_generic_kernel<OUT_U8, 1024, BF16><<<grid, threads, CROP_RAW_BYTES, st>>>(images, B, H, W, geom, glist, gcount, T, nbands, f4,
-                                                                                    swap_rb, lut, outf, outb);
-    }
+    auto gfn = bpc_crop_generic_kernel<OUT_U8, 256, BF16>;
+    if constexpr (!BF16)                                        // bfloat16 runs beside the CTA kernel only: T <= 256
+        if (threads > 256) gfn = bpc_crop_generic_kernel<OUT_U8, 1024>;
+    e = cudaFuncSetAttribute(gfn, cudaFuncAttributeMaxDynamicSharedMemorySize, CROP_RAW_BYTES);
+    if (e != cudaSuccess) return (int)e;
+    gfn<<<grid, threads, CROP_RAW_BYTES, st>>>(images, B, H, W, geom, glist, gcount, T, nbands, f4, swap_rb, lut, outf, outb);
     BPC_LAUNCH_CHECK();
     return BPC_OK;
 }

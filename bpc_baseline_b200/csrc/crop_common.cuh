@@ -5,9 +5,7 @@
 #include <cuda.h>
 
 #include <stdlib.h>
-#include <string.h>
 
-#include <mutex>
 #include <type_traits>
 
 #include "common.cuh"
@@ -24,8 +22,7 @@ constexpr int WARPK_WARPS = 8;
 constexpr int LUT_STRIDE = 257;              // shared-memory LUT: 256 entries + the normalised fill value per output channel
 constexpr int LUT_SMEM = 3200;               // 3 * 257 floats, padded to a multiple of 128 (TMA destinations follow)
 constexpr int WARPK_SMEM = WARPK_WARPS * WARP_SMEM + LUT_SMEM;
-constexpr int STREAM_ROWS = 8;               // streaming class-1 path: source rows per ring slot (= one TMA box)
-constexpr int STREAM_MAX_PITCH = 288;        // widest staging pitch of a class-1 strip (32 columns at scale < 2 need <= 256)
+constexpr int CTA_ROWS = 8;                  // CTA kernel: source rows per ring slot (= one TMA box); per-source-row records come in whole slots
 constexpr int YSRC_PAD = 16;                 // per-source-row table: zero entries behind the last row (whole slots run to completion)
 static_assert(LUT_SMEM % 128 == 0 && LUT_SMEM >= 3 * LUT_STRIDE * 4, "LUT block");
 // descriptors per ROI: x axis ds float4, y axis ds + 8 float4 (class 1 reads the y block as 2*ds + 16 float2 source-row records),
@@ -49,20 +46,13 @@ struct RoiGeom {                             // 88 bytes, workspace
 };
 static_assert(sizeof(RoiGeom) == 88, "RoiGeom layout");
 
-// 2-D tensor maps over the image pool seen as [B*H rows][W*3/4 uint32] (only when W*3 is a multiple of 16): one map
-// per staging pitch, box = {pitch / 4 words, 4 rows} (2 rows for the two widest), so one TMA instruction stages four
-// source rows of a strip instead of one bulk copy per row; rows / columns beyond the pool are zero-filled by the TMA
-// unit, which removes the guarded tail path.
+// L2 promotion of the CTA kernel's tensor maps (crop_cta.cu)
 #ifndef BPC_L2_PROMO
 #define BPC_L2_PROMO CU_TENSOR_MAP_L2_PROMOTION_L2_128B
 #endif
-constexpr int N_TMAPS = 15;
-constexpr int N_TMAPS8 = 8;                  // 8-row boxes for the streaming class-1 path: pitches 64 .. 288
-struct TmapSet { CUtensorMap m[N_TMAPS]; CUtensorMap m8[N_TMAPS8]; };
-__host__ __device__ __forceinline__ int tmap_pitch(int need) { return need <= 448 ? (need < 64 ? 64 : ((need + 31) & ~31)) : ((need + 63) & ~63); }
-__host__ __device__ __forceinline__ int tmap_index(int pitch) { return pitch <= 448 ? (pitch - 64) / 32 : 13 + (pitch - 512) / 64; }
-__host__ __device__ __forceinline__ int tmap_rows(int pitch) { return pitch <= 448 ? 4 : 2; }
-constexpr int TMAP_MAX_PITCH = 576;
+// Widest staging row of a class-4 strip on the warp kernel (four ring slots of at least three rows fit 2 * WARP_BUF); the CTA
+// kernel takes only pools whose row pitch is at least this wide
+constexpr int WARP_MAX_PITCH = 576;
 
 struct YDesc {                               // generic kernel, per output row of the band
     int start;

@@ -25,7 +25,6 @@ namespace bpc {
 //   class 3 (fixed-point bilinear, the box grows): per OUTPUT row (b0, b1, second source row, first source row); an output row
 //            is emitted as soon as the slot holding its second source row has landed -- its first row is the previous output
 //            row's first or second row, whose horizontal pass is still in registers.
-constexpr int CTA_ROWS = 8;                  // source rows per ring slot (= one TMA box)
 // ring slots and resident CTAs per SM: the T = 224 float instantiation (the benchmark's) runs 4 CTAs/SM (8 warps, 63 registers,
 // three slots: 55 KB of shared memory), which buys classes 3 and 4 latency hiding (0.66 -> 0.70, 0.67 -> 0.69) and leaves class 1
 // where it was; the run-time-T and T = 256 instantiations (up to 9 warps) keep four slots and 3 CTAs/SM

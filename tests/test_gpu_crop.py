@@ -88,7 +88,7 @@ def test_random_boxes_all_regimes_full_res(T):
 @pytest.mark.parametrize('T,width', [(224, 1920), (64, 1920), (256, 1920), (128, 3840), (256, 1918), (100, 1913)])
 def test_large_boxes_four_to_six_taps(T, width):
     """Boxes of 2T .. 5.3T: the 4 / 5 / 6-tap class (source-row records in the CTA kernel, wide rows by 1-D bulk copies; the
-    row-streaming ring of the per-strip kernel for unaligned pitches) and, beyond scale 5, the generic kernel.  width 1920 / 3840:
+    row-streaming ring of the per-strip kernel on the pools the CTA kernel does not take) and, beyond scale 5, the generic kernel.  width 1920 / 3840:
     image pitch a multiple of 16 bytes (CTA kernel, 2-D TMA staging); 1918 / 1913: the per-strip kernel's 1-D bulk-copy path."""
     from bpc_baseline_b200 import batched, synth
     imgs = synth.make_images(2, seed=9, width=width, height=1080)
@@ -143,8 +143,9 @@ def test_target_sizes_above_256(T):
 
 @pytest.mark.parametrize('width', [16, 64, 176, 192, 208, 256])
 def test_small_images_with_16_byte_pitch(width):
-    """Image rows of 48 .. 768 bytes, all multiples of 16: below 576 bytes (the widest staging box) the 1-D copy path is
-    used, from 192 px on the 2-D tensor-map path whose boxes may then be as wide as, or wider than, what is left of a row."""
+    """Image rows of 48 .. 768 bytes, all multiples of 16: the per-strip kernel's 1-D copies at T = 224 and below 576 bytes
+    (WARP_MAX_PITCH); from 192 px on at T = 64 the CTA kernel, whose 2-D tensor-map boxes may then be as wide as, or wider
+    than, what is left of a row."""
     from bpc_baseline_b200 import batched, synth
     H = 120
     imgs = synth.make_images(3, seed=12, width=width, height=H)

@@ -3,7 +3,7 @@
 Which kernel and which template instantiation crops a ROI is decided at run time (``launch_crop`` in csrc/crop.cu,
 ``crop_cta_launch`` in csrc/crop_cta.cu) from the pool width W, the target size T, the output type and ``swap_rb``:
 
-    aligned = 3 W % 16 == 0 and 3 W >= 576                      (2-D tensor-map staging possible)
+    aligned = 3 W % 16 == 0 and 3 W >= 576                      (16-byte row pitch, at least WARP_MAX_PITCH)
     use_cta = aligned and T <= 256 and 3 W >= cta_pitch_max(T)   (cta_pitch_max(224) = 1408, (256) = 1600)
     TT      = T if T in (224, 256) else 0                        (compile-time target size of the float kernels)
 
@@ -13,11 +13,11 @@ Which kernel and which template instantiation crops a ROI is decided at run time
       bf16  <0, swap>                                               for u8, f32 and (NTH = 256 only) bf16
       u8    <0>
     else:    bpc_crop_warp_kernel
-      f32   <TT, aligned, swap>
-      u8    <0, aligned>
+      f32   <TT, swap>
+      u8    <0>
       bf16  refused (BPC_EUNSUPPORTED)
 
-That is 9 CTA, 14 warp and 5 generic instantiations (``generic<bf16, 1024>`` is compiled but cannot run: bf16 needs
+That is 9 CTA, 7 warp and 5 generic instantiations (``generic<bf16, 1024>`` is compiled but cannot run: bf16 needs
 T <= 256).  ``TABLE`` lists the cells (kernel, instantiation, class) they make: 4 classes on the CTA and warp kernels,
 class 2 on the generic one.  ``crop_plan`` / ``roi_class`` restate the dispatch and the prep kernel's classification
 (``bpc_crop_prep_kernel``) in Python.  After every launch the tests read what the prep kernel actually did from the crop
@@ -40,7 +40,7 @@ import torch
 from oracle import crop as ocrop
 from tests.gpu_util import to_dev
 
-TMAP_MAX_PITCH = 576
+WARP_MAX_PITCH = 576
 CTA_MAX_T = 256
 MAX_ROI_WIDTH = 8192
 GEOM_BYTES = 88                  # sizeof(RoiGeom); cls is the int32 at byte 68
@@ -70,13 +70,13 @@ def ws_off_count(R, T):
 
 
 def pool_flags(W, T):
-    aligned = (3 * W) % 16 == 0 and 3 * W >= TMAP_MAX_PITCH
+    aligned = (3 * W) % 16 == 0 and 3 * W >= WARP_MAX_PITCH
     return aligned, aligned and T <= CTA_MAX_T and 3 * W >= cta_pitch_max(T)
 
 
 def crop_plan(W, T, out_type, swap):
     """{class: (kernel, instantiation)} of one launch, or None where the call is refused (bf16 off the CTA path)."""
-    aligned, use_cta = pool_flags(W, T)
+    use_cta = pool_flags(W, T)[1]
     sw = 'swap' if swap else 'keep'
     tt = T if T in (224, 256) else 0
     if out_type == 'bf16' and not use_cta:
@@ -84,8 +84,7 @@ def crop_plan(W, T, out_type, swap):
     if use_cta:
         fast = ('cta', {'f32': f'f32<{tt},{sw}>', 'bf16': f'bf16<0,{sw}>', 'u8': 'u8<0>'}[out_type])
     else:
-        al = 'aligned' if aligned else 'unaligned'
-        fast = ('warp', f'f32<{tt},{al},{sw}>' if out_type == 'f32' else f'u8<0,{al}>')
+        fast = ('warp', f'f32<{tt},{sw}>' if out_type == 'f32' else 'u8<0>')
     nth = 256 if (T + 31) // 32 * 32 <= 256 else 1024
     return {0: fast, 1: fast, 3: fast, 4: fast, 2: ('generic', f'{out_type}<{nth}>')}
 
@@ -95,11 +94,10 @@ def _table():
     for sw in ('swap', 'keep'):
         for tt in (224, 256, 0):
             cells |= {('cta', f'f32<{tt},{sw}>', c) for c in (0, 1, 3, 4)}
-            for al in ('aligned', 'unaligned'):
-                cells |= {('warp', f'f32<{tt},{al},{sw}>', c) for c in (0, 1, 3, 4)}
+            cells |= {('warp', f'f32<{tt},{sw}>', c) for c in (0, 1, 3, 4)}
         cells |= {('cta', f'bf16<0,{sw}>', c) for c in (0, 1, 3, 4)}
     cells |= {('cta', 'u8<0>', c) for c in (0, 1, 3, 4)}
-    cells |= {('warp', f'u8<0,{al}>', c) for al in ('aligned', 'unaligned') for c in (0, 1, 3, 4)}
+    cells |= {('warp', 'u8<0>', c) for c in (0, 1, 3, 4)}
     cells |= {('generic', f'{o}<{n}>', 2) for o, n in (('u8', 256), ('f32', 256), ('bf16', 256), ('u8', 1024), ('f32', 1024))}
     return frozenset(cells)
 
@@ -134,8 +132,8 @@ def _records_bad(h, new_h, scale_y, cap, maxtaps):
     return False
 
 
-def roi_class(w, h, T, use_cta, aligned):
-    """Class bpc_crop_prep_kernel gives a w x h box (crop.cu:103-137 plus the record check of classes 1 and 4):
+def roi_class(w, h, T, use_cta):
+    """Class bpc_crop_prep_kernel gives a w x h box (crop.cu:102-136 plus the record check of classes 1 and 4):
     0 rejected, 1 area with scale < 2 (or exactly 1), 3 grow, 4 area with 4..6 taps, 2 the generic kernel."""
     if w <= 0 or h <= 0 or w > MAX_ROI_WIDTH:
         return 0
@@ -157,12 +155,12 @@ def roi_class(w, h, T, use_cta, aligned):
         seg_px = int(31.0 * sx) + math.ceil(sx) + 3
         pitch_max = ((3 * seg_px + 46) >> 4) << 4
         taps6 = math.ceil(sx) + 1 <= 6 and math.ceil(sy) + 1 <= 6
-        cls = 4 if taps6 and (use_cta or pitch_max <= TMAP_MAX_PITCH) else 2
+        cls = 4 if taps6 and (use_cta or pitch_max <= WARP_MAX_PITCH) else 2
     else:
         cls = 2
     if cls == 4 and use_cta and _records_bad(h, new_h, sy, 2 * ydesc_stride(T), 6):
         cls = 2
-    if cls == 1 and aligned and _records_bad(h, new_h, sy, 2 * desc_stride(T) + 16, 3):
+    if cls == 1 and use_cta and _records_bad(h, new_h, sy, 2 * desc_stride(T) + 16, 3):
         cls = 2
     return cls
 
@@ -171,8 +169,7 @@ def box_class(box, B, H, W, T):
     img, x1, y1, x2, y2 = (int(v) for v in box)
     if not (0 <= img < B and x1 >= 0 and y1 >= 0 and x2 <= W and y2 <= H):
         return 0
-    aligned, use_cta = pool_flags(W, T)
-    return roi_class(x2 - x1, y2 - y1, T, use_cta, aligned)
+    return roi_class(x2 - x1, y2 - y1, T, pool_flags(W, T)[1])
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -180,10 +177,10 @@ def box_class(box, B, H, W, T):
 # ----------------------------------------------------------------------------------------------------------------------
 TS = (1, 2, 3, 31, 33, 97, 100, 224, 255, 256, 257)
 MATRIX = (
-    [(1920, T) for T in TS]                                         # CTA (T <= 256), aligned warp at T = 257
-    + [(1918, T) for T in TS]                                       # unaligned warp (pitch 5754)
-    + [(448, 224), (448, 256), (512, 256), (320, 160), (192, 97)]   # aligned warp: 16-byte pitch below cta_pitch_max(T)
-    + [(1913, 224), (1913, 33)]                                     # unaligned warp, another misalignment step
+    [(1920, T) for T in TS]                                         # CTA (T <= 256), warp on a 16-byte pitch at T = 257
+    + [(1918, T) for T in TS]                                       # warp (pitch 5754, not a multiple of 16)
+    + [(448, 224), (448, 256), (512, 256), (320, 160), (192, 97)]   # warp: 16-byte pitch below cta_pitch_max(T)
+    + [(1913, 224), (1913, 33)]                                     # warp, another misalignment step
     + [(176, 3), (176, 33), (176, 224), (176, 256)]                 # 528-byte pitch: a multiple of 16, below 576
 )
 POOL_H, POOL_B = 1400, 2
@@ -247,7 +244,7 @@ def test_dispatch_restatement_table_and_boundaries():
                     plan = crop_plan(W, T, out, swap)
                     if plan is not None:
                         reached |= {(*plan[c], c) for c in plan}
-    assert reached == TABLE and len(TABLE) == 36 + 56 + 5
+    assert reached == TABLE and len(TABLE) == 36 + 28 + 5
     assert cta_pitch_max(224) == 1408 and cta_pitch_max(256) == 1600
     kern = lambda W, T: crop_plan(W, T, 'f32', True)[1][0]
     assert [kern(W, 224) for W in (176, 192, 464, 480, 601)] == ['warp', 'warp', 'warp', 'cta', 'warp']
@@ -272,10 +269,10 @@ def test_matrix_plan_reaches_every_cell():
 
 def test_roi_class_rounding_ties():
     # 6 x 3 and 2 x 1 at T = 1: the short side is 0.5 -> 0 (rejected); at T = 3: 1.5 -> 2; 2 x 1 at T = 7: 3.5 -> 4
-    assert [roi_class(6, 3, 1, False, False), roi_class(2, 1, 1, False, False)] == [0, 0]
+    assert [roi_class(6, 3, 1, False), roi_class(2, 1, 1, False)] == [0, 0]
     assert ocrop.letterbox_geometry(3, 6, 3)[1:3] == (3, 2) and ocrop.letterbox_geometry(1, 2, 7)[1:3] == (7, 4)
-    assert roi_class(6, 3, 3, False, False) == 4 and roi_class(2, 1, 3, False, False) == 3
-    assert roi_class(8192, 600, 224, True, True) == 2 and roi_class(8193, 600, 224, True, True) == 0
+    assert roi_class(6, 3, 3, False) == 4 and roi_class(2, 1, 3, False) == 3
+    assert roi_class(8192, 600, 224, True) == 2 and roi_class(8193, 600, 224, True) == 0
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -370,7 +367,7 @@ def _matrix_case(W, T):
         assert np.array_equal(status.cpu().numpy(), st_want)
         bad = [r for r in range(R) if not np.array_equal(out[r], canvas[r])]
         assert not bad, ('u8', fill, [tuple(rois[r]) for r in bad[:6]])
-    aligned, use_cta = pool_flags(W, T)
+    use_cta = pool_flags(W, T)[1]
     for swap in (False, True):
         for fill, lk in (((0, 128, 255), 'rand'), ((7, 200, 31), 'norm'), ((255, 255, 255), 'rand')):
             canvas, st_want = ref[fill]
@@ -430,8 +427,8 @@ def test_bf16_refused_exactly_off_the_cta_path(W, T):
 @pytest.mark.parametrize('W,T', [(1918, 100), (448, 224), (176, 33), (1920, 300), (1920, 97)])
 def test_device_count_on_every_kernel(W, T):
     """n_rois with a nonzero roi_first falling inside one launch: rows at or beyond the count keep the sentinel (output
-    and status), their class is -1, and the rows below it are correct -- on the warp kernel (aligned / unaligned, rejected
-    boxes among the skipped rows), the generic kernel (class-2 boxes on both sides of the count) and the CTA kernel."""
+    and status), their class is -1, and the rows below it are correct -- on the warp kernel (16-byte and other pitches,
+    rejected boxes among the skipped rows), the generic kernel (class-2 boxes on both sides of the count) and the CTA kernel."""
     from bpc_baseline_b200 import batched
     imgs = _pool(W, POOL_H, POOL_B, 40 + W % 97)
     rois = matrix_boxes(W, POOL_H, POOL_B, T, seed=(W, T, 1))

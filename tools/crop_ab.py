@@ -4,6 +4,9 @@ so that a faster variant whose bytes differ is caught in the same run.
 
     python tools/crop_ab.py [--reps N] libA.so libB.so ...      # paths relative to the repo root; each runs in its own process
 
+Environment: RANGES (box side ranges in px), T (target size, default 224), POOL_W (pool width in px, default 3840; boxes are
+clipped to it).  The crop count scales as 1 / T^2, so every T writes about the output bytes of 16384 crops at T = 224.
+
 Build variants here first (nvcc cross-compiles):  python -c "from bpc_baseline_b200 import build; build.build(True, defines=['X'], out='...')"
 """
 import json
@@ -13,6 +16,8 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 RANGES = tuple(tuple(int(v) for v in r.split('-')) for r in os.environ.get('RANGES', '60-400,300-900,32-96').split(','))
+T = int(os.environ.get('T', 224))
+POOL_W = int(os.environ.get('POOL_W', 3840))
 
 
 def one(reps):
@@ -23,13 +28,13 @@ def one(reps):
     import bench_configs as bc
     from bpc_baseline_b200 import batched, pipeline, synth
     out = {}
-    R, T, B = 16384, 224, 8
-    images = bc.dev(synth.make_images(B * 3, seed=44))
+    R, B = 16384 * 224 * 224 // (T * T), 8
+    images = bc.dev(synth.make_images(B * 3, seed=44, width=POOL_W))
     buf = torch.empty((R, 3, T, T), dtype=torch.float32, device='cuda')
     for lo, hi in RANGES:
         rng = np.random.default_rng([44, lo, hi, T])
-        w = rng.integers(lo, hi, R); h = rng.integers(lo, hi, R)
-        x1 = (rng.random(R) * (synth.IMG_W - w)).astype(np.int64); y1 = (rng.random(R) * (synth.IMG_H - h)).astype(np.int64)
+        w = np.minimum(rng.integers(lo, hi, R), POOL_W); h = rng.integers(lo, hi, R)
+        x1 = (rng.random(R) * (POOL_W - w)).astype(np.int64); y1 = (rng.random(R) * (synth.IMG_H - h)).astype(np.int64)
         rois = np.stack([rng.integers(0, B * 3, R), x1, y1, x1 + w, y1 + h], axis=1).astype(np.int32)
         drois = bc.dev(rois)
         buf.zero_()
