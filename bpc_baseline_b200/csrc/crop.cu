@@ -26,6 +26,8 @@
 //                     source rows streamed through shared memory in chunks (boxes as large as the image).
 // The dominant traffic is the float32 output (3*T*T*4 B per ROI): each warp stores 128 contiguous bytes per
 // plane and row; padding rows are written with 16-byte stores.
+#include <cooperative_groups.h>
+
 #include <type_traits>
 
 #include "crop_common.cuh"
@@ -196,6 +198,149 @@ bpc_crop_prep_kernel(const uint8_t* __restrict__ images, int B, int H, int W, co
         else if (use_cta && g.cls != -1) list1[atomicAdd(gcount + 8, 1)] = roi;     // classes 0, 1, 3, 4: the CTA kernel's list
         geom[roi] = g;
     }
+}
+
+// ------------------------------------------------------------------------------------------------------
+// order of the CTA kernel's list: crops by their first source row in the pool
+// ------------------------------------------------------------------------------------------------------
+// The prep kernel appends the list in about ROI order, which for a batch of scenes is scene order: when scenes share
+// captures (a pool of images) or their detections overlap, a source line is needed again only hundreds of crops later,
+// after more output than the 126 MB L2 holds has streamed through it.  Sorted by first source row (image * H + y1), the
+// crops in flight read a narrow band of the pool and the repeated lines come from L2.  Outputs do not change: each crop
+// writes its own slot only, the order decides when it runs.
+// Only a list whose crops read more source pixels than the pool holds is reordered: every pool pixel is then read more
+// than once on average, so the crops must share lines.  Where they share less (boxes that do not overlap, small boxes in
+// a large pool) the new order buys nothing and scatters the output slots being written (3-4 % slower, DESIGN.md 3.2),
+// and the list stays as prep wrote it.  counters[9] = 1 marks a reordered list (the CTA kernel then keeps the source
+// lines in L2 with an evict-last policy).
+// One cluster of ORDER_CTAS CTAs, each over a slice of the list (one CTA over the whole list took 40 us per 16 384 entries,
+// the cluster 15 us; DESIGN.md 3.2): per CTA a shared-memory histogram over buckets of
+// 2^shift rows (shift the least that leaves at most ORDER_BUCKETS of them in [0, B H)); through distributed shared memory
+// every CTA adds up the cluster's counts per bucket and those of the lower-ranked CTAs, scans them and scatters its entries
+// into the unused tail of the generic list (glist[gcount, R) holds at least n1 entries, as gcount + n1 <= R); after a
+// cluster barrier each CTA copies its slice back into list1.  Ties (crops in one bucket) fall in any order.
+constexpr int ORDER_CTAS = 8;
+constexpr int ORDER_THREADS = 1024;
+constexpr int ORDER_BUCKETS = 4096;
+constexpr int ORDER_BATCH = 6;                // list entries per thread with their loads in flight together
+
+__global__ void __cluster_dims__(ORDER_CTAS, 1, 1) __launch_bounds__(ORDER_THREADS)
+bpc_crop_order_kernel(const uint8_t* __restrict__ images, int B, int H, int W, const RoiGeom* __restrict__ geom,
+                      int32_t* __restrict__ list1, int32_t* __restrict__ counters, int32_t* __restrict__ glist) {
+    namespace cg = cooperative_groups;
+    __shared__ __align__(16) int cnt[ORDER_BUCKETS];   // this CTA's entries per bucket (read by the whole cluster)
+    __shared__ int pos[ORDER_BUCKETS];            // next list slot of this CTA's entries per bucket
+    __shared__ int wsum[ORDER_THREADS / 32];
+    __shared__ unsigned long long wpx[ORDER_THREADS / 32], s_px;
+    const int n = counters[8];
+    if (n < 2) return;
+    cg::cluster_group cluster = cg::this_cluster();
+    const int rank = (int)cluster.block_rank();
+    const int per = (n + ORDER_CTAS - 1) / ORDER_CTAS;
+    const int lo = min(n, rank * per), hi = min(n, lo + per);
+    int32_t* tmp = glist + counters[0];
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const unsigned long long base = (unsigned long long)(uintptr_t)images, rowstride = (unsigned long long)W * 3ull;
+    const unsigned long long rows = (unsigned long long)B * H;
+    const double inv_rowstride = 1.0 / (double)rowstride;
+    const int shift = max(0, 64 - __clzll((long long)rows - 1) - 12);          // (B H - 1) >> shift < ORDER_BUCKETS
+    for (int b = tid; b < ORDER_BUCKETS; b += ORDER_THREADS) cnt[b] = 0;
+    __syncthreads();
+    // visit(roi, bucket, w h) for the entries [lo, hi) (w h = 0 unless `area`).  First source row = (src - images) / (3 W):
+    // the double quotient is within one row of the exact one (no 64-bit division).  A rejected box (class 0, src = 0) has
+    // no source rows and goes to bucket 0.
+    auto pass = [&](bool area, auto&& visit) {
+        for (int i0 = lo; i0 < hi; i0 += ORDER_THREADS * ORDER_BATCH) {
+            int roi[ORDER_BATCH];
+            unsigned long long src[ORDER_BATCH];
+            int2 wh[ORDER_BATCH];
+#pragma unroll
+            for (int k = 0; k < ORDER_BATCH; ++k) {
+                const int i = i0 + k * ORDER_THREADS + tid;
+                roi[k] = i < hi ? list1[i] : -1;
+            }
+#pragma unroll
+            for (int k = 0; k < ORDER_BATCH; ++k) {
+                src[k] = roi[k] >= 0 ? geom[roi[k]].src : 0ull;
+                wh[k] = roi[k] >= 0 && area ? *reinterpret_cast<const int2*>(&geom[roi[k]].w) : make_int2(0, 0);
+            }
+#pragma unroll
+            for (int k = 0; k < ORDER_BATCH; ++k) {
+                if (roi[k] < 0) continue;
+                int b = 0;
+                if (src[k]) {
+                    const unsigned long long off = src[k] - base;
+                    unsigned long long row = (unsigned long long)((double)off * inv_rowstride);
+                    if (row * rowstride > off) --row;
+                    else if ((row + 1) * rowstride <= off) ++row;
+                    b = (int)(row >> shift);
+                }
+                visit(roi[k], b, src[k] ? (unsigned long long)wh[k].x * (unsigned long long)wh[k].y : 0ull);
+            }
+        }
+    };
+    unsigned long long px = 0ull;                                   // source pixels of this thread's crops
+    pass(true, [&](int, int b, unsigned long long a) { atomicAdd(&cnt[b], 1); px += a; });
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) px += __shfl_down_sync(0xffffffffu, px, d);
+    if (lane == 0) wpx[wid] = px;
+    __syncthreads();
+    if (tid == 0) {
+        unsigned long long t = 0ull;
+        for (int w = 0; w < ORDER_THREADS / 32; ++w) t += wpx[w];
+        s_px = t;
+    }
+    cluster.sync();                                                 // every CTA's counts and pixel sum are complete
+    unsigned long long list_px = 0ull;
+    for (int r = 0; r < ORDER_CTAS; ++r) list_px += *cluster.map_shared_rank(&s_px, r);
+    if (list_px <= rows * (unsigned long long)W) {                  // the same decision in every CTA
+        cluster.sync();                                             // no CTA reads another's shared memory after this
+        return;
+    }
+    constexpr int PER = ORDER_BUCKETS / ORDER_THREADS;
+    static_assert(PER * ORDER_THREADS == ORDER_BUCKETS && ORDER_THREADS == 1024, "four buckets per thread, 32 warps");
+    int c[PER], below[PER], s = 0;
+#pragma unroll
+    for (int k = 0; k < PER; ++k) c[k] = below[k] = 0;
+    for (int r = 0; r < ORDER_CTAS; ++r) {                          // one 16-byte remote load per rank and thread
+        const int4 v = reinterpret_cast<const int4*>(cluster.map_shared_rank(cnt, r))[tid];
+        const int vk[PER] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < PER; ++k) {
+            c[k] += vk[k];
+            if (r < rank) below[k] += vk[k];
+        }
+    }
+    cluster.sync();                                                 // no CTA reads another's shared memory after this
+#pragma unroll
+    for (int k = 0; k < PER; ++k) s += c[k];
+    int incl = s;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += v;
+    }
+    if (lane == 31) wsum[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+        const int v = wsum[lane];
+        int iv = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int u = __shfl_up_sync(0xffffffffu, iv, d);
+            if (lane >= d) iv += u;
+        }
+        wsum[lane] = iv - v;
+    }
+    __syncthreads();
+    int run = wsum[wid] + incl - s;
+#pragma unroll
+    for (int k = 0; k < PER; ++k) { pos[tid * PER + k] = run + below[k]; run += c[k]; }
+    __syncthreads();
+    pass(false, [&](int roi, int b, unsigned long long) { tmp[atomicAdd(&pos[b], 1)] = roi; });
+    cluster.sync();                                                 // the whole list is in tmp (release / acquire over the cluster)
+    for (int i = lo + tid; i < hi; i += ORDER_THREADS) list1[i] = tmp[i];
+    if (rank == 0 && tid == 0) counters[9] = 1;
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -815,7 +960,7 @@ static int launch_crop(const uint8_t* images, int B, int H, int W, const int32_t
     RoiGeom* geom = (RoiGeom*)wsb;
     float4* xdesc = (float4*)(wsb + ws_off_xdesc(R));
     float4* ydesc = (float4*)(wsb + ws_off_ydesc(R, T));
-    int32_t* gcount = (int32_t*)(wsb + ws_off_count(R, T));   // [0] generic-list length, [4] warp-item counter, [8] CTA-list length, [12] its work counter
+    int32_t* gcount = (int32_t*)(wsb + ws_off_count(R, T));   // [0] generic-list length, [4] warp-item counter, [8] CTA-list length, [9] 1 if that list was reordered, [12] its work counter
     int32_t* wcount = gcount + 4;
     int32_t* glist = gcount + 16;
     int32_t* list1 = glist + R;
@@ -830,6 +975,8 @@ static int launch_crop(const uint8_t* images, int B, int H, int W, const int32_t
     BPC_LAUNCH_CHECK();
     const uchar4 f4 = make_uchar4(fill[0], fill[1], fill[2], 0);
     if (use_cta) {                                        // every fast-class crop is on the CTA kernel's list
+        bpc_crop_order_kernel<<<ORDER_CTAS, ORDER_THREADS, 0, st>>>(images, B, H, W, geom, list1, gcount, glist);
+        BPC_LAUNCH_CHECK();
         const int rc = crop_cta_launch(OUT_U8 ? 1 : (BF16 ? 2 : 0), images, B, H, W, geom, xdesc, ydesc, list1, gcount, R, T, f4, swap_rb, lut,
                                        outf, outb, st);
         if (rc != BPC_OK) return rc;

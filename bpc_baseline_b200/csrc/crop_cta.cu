@@ -87,6 +87,11 @@ bpc_crop_cta_kernel(const uint8_t* __restrict__ images, int B, int H, int W, con
     if (wid == NS) {
         // ------------------------------------ producer ------------------------------------
         if (lane != 0) return;
+        // a list ordered by source row (bpc_crop_order_kernel) reads each source line again a few crops later: keep the lines in
+        // L2 while the output streams past (evict-last; on boxes that do not overlap, which share nothing, it measured slower)
+        const bool keep_src = counters[9] != 0;
+        unsigned long long src_policy;
+        asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(src_policy));
         int idx = atomicAdd(work, 1);
         unsigned cg = 0;                                            // slots filled so far
         for (int hi = 0;; ++hi) {
@@ -122,8 +127,12 @@ bpc_crop_cta_kernel(const uint8_t* __restrict__ images, int B, int H, int W, con
                     const unsigned j = cg % CTA_NSLOT;
                     if (cg >= CTA_NSLOT) mbar_wait(empty_s + 8 * j, ((cg / CTA_NSLOT) - 1) & 1);
                     mbar_expect_tx(full_s + 8 * j, (unsigned)(CTA_ROWS * pitch));
-                    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                                 :: "r"(ring_s + j * slot_bytes), "l"(map), "r"(x8), "r"(row0 + c * CTA_ROWS), "r"(full_s + 8 * j) : "memory");
+                    if (keep_src)
+                        asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], %5;"
+                                     :: "r"(ring_s + j * slot_bytes), "l"(map), "r"(x8), "r"(row0 + c * CTA_ROWS), "r"(full_s + 8 * j), "l"(src_policy) : "memory");
+                    else
+                        asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+                                     :: "r"(ring_s + j * slot_bytes), "l"(map), "r"(x8), "r"(row0 + c * CTA_ROWS), "r"(full_s + 8 * j) : "memory");
                 }
             } else {
                 // wide class-4 crops (rows of up to 5 T pixels): rps rows per slot, one 1-D bulk copy each, clipped to the pool
